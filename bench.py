@@ -175,9 +175,9 @@ def run_ours(args):
         """the whole round on resident inputs: realign, score cut, consensus (N > 1: the sharded protocol,
         2 all-reduces + 1 small all-gather over NCCL on the library's stream; same work per read at every N)"""
         g.reset_dropped()                               # every timed step starts from the same state
-        cons = g.iterate_resident()[0] if world == 1 else S.resident()[0]
+        cons, cut, _ = g.iterate_resident() if world == 1 else S.resident()
         launches["n"] += g.last_timing()["launches"]
-        return cons
+        return cons, cut
 
     # pinned host buffers for the end-to-end path
     def pin(a):
@@ -215,7 +215,7 @@ def run_ours(args):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
     sampler = ClockSampler(local) if rank == 0 else None      # nvidia-smi needs a few hundred ms to start: launched before the warm-up
     for _ in range(max(args.warmup, 3)):
-        cons = step_resident()
+        cons, _ = step_resident()
     tim = g.last_timing()
     barrier()
     if sampler:
@@ -230,10 +230,16 @@ def run_ours(args):
         flush.zero_()                       # L2 flush between timed iterations (outside the timed events)
         barrier()
         ev[k][0].record(lib_stream)
-        cons = step_resident()
+        cons, cut = step_resident()
         ev[k][1].record(lib_stream)
         torch.cuda.synchronize()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # what a caller of the round receives: the consensus and the cut here, the per-read alignment and the run lists
+        # from the device (miagpu_get_alignment + miagpu_get_runs_packed), before the per-class timing below overwrites them
+        total_runs = g.get_runs_packed()[0]
+        packed = g.get_runs_packed(None, np.zeros(total_runs, np.uint16))[2]
+        dumped = {"consensus": cons, "score_cut": cut, "aln": g.get_alignment(), "runs": packed}
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = float(sum(step_ms))
     # resident realigns on the measurement path (one width class after the other, events around each) just to read the
@@ -262,6 +268,10 @@ def run_ours(args):
     barrier()
     clocks = sampler.stop() if sampler else None
     e2e_total = float(sum(e2e_times))
+    if args.dump_outputs and rank == 0:
+        e2e = {"consensus": cons_e2e, "aln": {k: v.numpy() for k, v in h_out.items()}, "dropped": dropped.numpy(),
+               "runs": h_packed[: packed_total["n"]].numpy().view(np.uint16)}
+        dump_outputs(args.dump_outputs, dumped, e2e, n)
 
     if world > 1:
         t = torch.tensor([total_ms, e2e_total], dtype=torch.float64, device="cuda")
@@ -374,6 +384,37 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_READS = 200_000            # per-read sample of --dump-outputs: 13 arrays, 2 x 24 run words and an index, at most 51 MB
+
+
+def _runs_of(packed, n_runs, idx):
+    """the packed run words of reads idx (sorted) out of a read-order packing with n_runs words per read"""
+    first = np.concatenate(([0], np.cumsum(n_runs, dtype=np.int64)))[idx]
+    lens = n_runs[idx].astype(np.int64)
+    start = np.concatenate(([0], np.cumsum(lens)))
+    return packed[np.repeat(first - start[:-1], lens) + np.arange(start[-1])]
+
+
+def dump_outputs(d, resident, e2e, n):
+    """--dump-outputs: what the last timed step of each arm handed back -- consensus (byte codes), score cut (slope, intercept),
+    per-read alignment and packed run lists, and from the end-to-end arm also the sticky dropped flags -- as DIR/<name>.npy,
+    float32 (float64 for the cut and the read indices).  The inputs are a function of the arguments, so two builds run with the
+    same arguments can be compared file by file.  Per-read arrays cover a fixed seeded sample of DUMP_READS reads when there
+    are more (read indices in reads.npy)."""
+    os.makedirs(d, exist_ok=True)
+    idx = np.arange(n) if n <= DUMP_READS else np.sort(np.random.default_rng(0).choice(n, DUMP_READS, replace=False))
+    out = {"reads": idx.astype(np.float64)}
+    for prefix, arm in (("", resident), ("e2e_", e2e)):
+        out[prefix + "consensus"] = np.frombuffer(arm["consensus"].encode(), np.uint8).astype(np.float32)
+        for k, v in arm["aln"].items():
+            out[prefix + k] = v[idx].astype(np.float32)
+        out[prefix + "runs"] = _runs_of(arm["runs"], arm["aln"]["n_runs"], idx).astype(np.float32)
+    out["score_cut"] = np.asarray(resident["score_cut"], np.float64)
+    out["e2e_dropped"] = e2e["dropped"][idx].astype(np.float32)
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), v)
+
+
 def parity_block(g, args, world, rank, local, ref, bases, off, rc, as_, ae, sm, cons_full):
     """Untimed: ties what was just measured to the CPU checker (oracle/_ref = the unmodified reference where it was built).
     (1) the first `--parity-reads` reads of rank 0's workload through one resident round on ONE GPU: every read's score / as /
@@ -444,9 +485,8 @@ def shaped_rounds(g, args, flush, lib_stream):
         for _ in range(3):
             g.reset_dropped()
             g.iterate_resident()
-        steps = max(3, args.steps // 2)
-        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
-        for k in range(steps):
+        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
+        for k in range(args.steps):
             flush.zero_()
             torch.cuda.synchronize()
             ev[k][0].record(lib_stream)
@@ -454,7 +494,7 @@ def shaped_rounds(g, args, flush, lib_stream):
             g.iterate_resident()
             ev[k][1].record(lib_stream)
             torch.cuda.synchronize()
-        ms = float(sum(a.elapsed_time(b) for a, b in ev)) / steps
+        ms = float(sum(a.elapsed_time(b) for a, b in ev)) / args.steps
         g.realign_resident()
         g.realign_resident()
         cells = g.last_timing()["dp_cells"]
@@ -774,7 +814,10 @@ def main():
     ap.add_argument("--no-shapes", action="store_true")
     ap.add_argument("--parity-reads", type=int, default=20000, help="prefix of rank 0's workload checked against the CPU reference")
     ap.add_argument("--pass1-unmasked-reads", type=int, default=1000000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
