@@ -2,6 +2,7 @@
  * compiled and run.  It is NOT the reference's CLI (SURVEY 8: out of scope): it covers the default assembly mode only
  *
  *     mia_gpu -r ref.fa -f reads.fq -s matrix.txt -m out [-c] [-k K] [-p 1|2] [-H cut | -S slope -N icpt] [-F] [-u | -U] [-A] [-D] [-h]
+ *             [-d damage.tsv]
  *
  * and exists to show (and test, tests/test_gpu_host_c.py) that the C ABI alone -- no Python, no torch -- reproduces
  * the reference's `.maln` files: reader (miagpu_fastx_*), matrices (miagpu_read_pssm), pass 1, score cut, one library
@@ -13,6 +14,9 @@
  * 2000 (strand_known = 0, mia.c:1653), never-cleared back pointers, slot-indexed sticky flags, and -D (mia.c:1614,
  * mia_main.c:120-174: miagpu_distant_retry).  -h (mia_main.c:497: the homopolymer discount in every alignment) is
  * miagpu_set_homopolymer.  -T, -C, -I are not handled here.
+ * -d FILE is an extension of this host, not a flag of the reference: the damage profile of the final round (miagpu_misincorporation,
+ * the misincorporation table of its `.maln` file by depth) as text, a header line depth / ref / read / count, then one line per cell
+ * of the [31][6][6] table in index order, bases as A C G T N -.  Without -d every output is what it is without the extension.
  * There is no CPU fallback: without a CUDA device miagpu_create fails and so does this program. */
 #define _POSIX_C_SOURCE 199309L
 #include <stdio.h>
@@ -69,6 +73,17 @@ static char* read_reference( const char* fn, char* id, char* desc, int* len_out 
   return seq;
 }
 
+/* -d: the table of miagpu_misincorporation as text */
+static void write_damage( const char* fn, const int64_t* t ) {
+  static const char code[] = "ACGTN-";
+  FILE* f = fopen( fn, "w" );
+  int c;
+  if ( !f ) { fprintf( stderr, "mia_gpu: cannot write %s\n", fn ); exit( 1 ); }
+  fprintf( f, "depth\tref\tread\tcount\n" );
+  for ( c = 0; c < MIAGPU_MISINC_INTS; c++ ) fprintf( f, "%d\t%c\t%c\t%lld\n", c / 36, code[c / 6 % 6], code[c % 6], (long long)t[c] );
+  if ( fclose( f ) != 0 ) { fprintf( stderr, "mia_gpu: cannot write %s\n", fn ); exit( 1 ); }
+}
+
 static unsigned char comp[256];
 static void init_comp( void ) {
   const char* a = "ACGTRYKMBDHVNSWacgtrykmbdhvnsw-";
@@ -123,7 +138,7 @@ static void filter_and_cull( miagpu_ctx* g, Fsdb* F ) {
 }
 
 int main( int argc, char** argv ) {
-  const char *ref_fn = NULL, *frag_fn = NULL, *mat_fn = NULL, *root = "assembly.maln.iter";
+  const char *ref_fn = NULL, *frag_fn = NULL, *mat_fn = NULL, *root = "assembly.maln.iter", *damage_fn = NULL;
   int circular = 0, k = -1, cons_code = 1, hard_cut = 0, final_only = 0, repeat_filt = 0, just_outer_coords = 1, i;
   int score_cut_set = 0, distant_ref = 0, n_unknown = 0, hp_special = 0;
   double user_slope = 200.0, user_icpt = 0.0;           /* DEF_S, DEF_N (params.h:36-37); -S / -N: mia_main.c:579-586 */
@@ -140,6 +155,10 @@ int main( int argc, char** argv ) {
     else if ( i + 1 < argc && !strcmp( argv[i], "-f" ) ) frag_fn = argv[++i];
     else if ( i + 1 < argc && !strcmp( argv[i], "-s" ) ) mat_fn = argv[++i];
     else if ( i + 1 < argc && !strcmp( argv[i], "-m" ) ) root = argv[++i];
+    else if ( !strcmp( argv[i], "-d" ) ) {
+      if ( i + 1 >= argc ) { fprintf( stderr, "mia_gpu: -d needs a file name (the damage profile of the final round)\n" ); return 2; }
+      damage_fn = argv[++i];
+    }
     else if ( i + 1 < argc && !strcmp( argv[i], "-k" ) ) k = atoi( argv[++i] );
     else if ( i + 1 < argc && !strcmp( argv[i], "-p" ) ) cons_code = atoi( argv[++i] );
     else if ( i + 1 < argc && !strcmp( argv[i], "-H" ) ) hard_cut = atoi( argv[++i] );
@@ -149,7 +168,8 @@ int main( int argc, char** argv ) {
   }
   if ( repeat_filt && ( hard_cut > 0 || score_cut_set || distant_ref ) ) { fprintf( stderr, "mia_gpu: -H / -S / -N / -D together with -u / -U are not handled by this host\n" ); return 2; }
   if ( !ref_fn || !frag_fn || !mat_fn ) {
-    fprintf( stderr, "usage: mia_gpu -r ref.fa -f reads.fa|fq -s matrix.txt [-m root] [-c] [-k K] [-p code] [-H cut] [-F] [-u|-U] [-A]\n" );
+    fprintf( stderr, "usage: mia_gpu -r ref.fa -f reads.fa|fq -s matrix.txt [-m root] [-c] [-k K] [-p code] [-H cut] [-F] [-u|-U] [-A]\n"
+                     "               [-d damage.tsv  (extension of this host: the final round's misincorporation table)]\n" );
     return 2;
   }
   init_comp();
@@ -372,6 +392,11 @@ int main( int argc, char** argv ) {
     { char* t = last; last = cons; cons = t; }
   }
   fprintf( stderr, converged ? "Assembly convergence after %d rounds\n" : "Assembly did not converge after %d rounds, quitting\n", iter );
+  if ( damage_fn ) {                                    /* the device still holds the final round */
+    static int64_t table[MIAGPU_MISINC_INTS];
+    CK( miagpu_misincorporation( g, table ) );
+    write_damage( damage_fn, table );
+  }
   fprintf( stderr, "mia_gpu: timing ms: init %.1f parse %.1f pass1 %.1f rounds %.1f write %.1f total %.1f\n", t_init, t_parse, t_pass1,
            t_rounds, t_write, now_ms() - t0 );
   miagpu_destroy( g );

@@ -2,7 +2,7 @@
  * thread per GPU, reads sharded contiguously in FSDB order, the consensus replicated, three NCCL collectives per round on the
  * library's own streams (the sequence INTEGRATION.md gives, compiled and run):
  *
- *     mia_gpu_mg -g N -r ref.fa -f reads.fq -s matrix.txt -m out [-c] [-k K] [-p 1|2] [-H cut | -S slope -N icpt] [-F]
+ *     mia_gpu_mg -g N -r ref.fa -f reads.fq -s matrix.txt -m out [-c] [-k K] [-p 1|2] [-H cut | -S slope -N icpt] [-F] [-d damage.tsv]
  *
  *       miagpu_shard_begin   -> ncclAllReduce( max_buf, MAX )        insert maxima, best scores, the ranks' integer sums
  *       miagpu_shard_fit     -> ncclAllGather( gather_send/recv )    block records of the regression's two chains
@@ -12,6 +12,8 @@
  * It writes the `.maln` files the one-GPU host (host/mia_gpu.c) and the reference write (tests/test_gpu_host_c.py runs both).
  * Sharded rounds give every read its own AlnSeqs and one sticky flag: input that needs the reference's pointer state (a read that
  * scores exactly 2000, -D) is refused here -- host/mia_gpu.c takes it.  -u / -U / -T / -h / -C / -I are not handled.
+ * -d FILE is an extension of this host, not a flag of the reference: the damage profile of the final round (miagpu_misincorporation
+ * of every GPU's context, summed here) in the text format of host/mia_gpu.c -d.  Without -d every output is what it is without it.
  * No CPU fallback: without CUDA devices miagpu_create fails and so does this program. */
 #define _POSIX_C_SOURCE 200809L
 #include <ctype.h>
@@ -89,6 +91,8 @@ typedef struct {
   char *last, *cons; int32_t* gaps; size_t cons_cap;
   int64_t run_total[MAX_GPUS]; int64_t *run_off, *run_off_r[MAX_GPUS]; uint16_t* packed[MAX_GPUS]; int64_t packed_cap[MAX_GPUS];
   int iter, converged, failed;
+  const char* damage_fn;
+  int64_t damage[MAX_GPUS][MIAGPU_MISINC_INTS];  /* -d: the final round's table of every rank */
   ncclComm_t comm[MAX_GPUS];
   pthread_barrier_t bar;
   double t_rounds, t_write;
@@ -103,6 +107,17 @@ static void init_comp( void ) {
   int i;
   for ( i = 0; i < 256; i++ ) comp[i] = 'N';
   for ( i = 0; a[i]; i++ ) comp[(unsigned char)a[i]] = (unsigned char)b[i];
+}
+
+/* -d: the table of miagpu_misincorporation as text (the format of host/mia_gpu.c) */
+static int write_damage( const char* fn, const int64_t* t ) {
+  static const char code[] = "ACGTN-";
+  FILE* f = fopen( fn, "w" );
+  int c;
+  if ( !f ) return 0;
+  fprintf( f, "depth\tref\tread\tcount\n" );
+  for ( c = 0; c < MIAGPU_MISINC_INTS; c++ ) fprintf( f, "%d\t%c\t%c\t%lld\n", c / 36, code[c / 6 % 6], code[c % 6], (long long)t[c] );
+  return fclose( f ) == 0;
 }
 
 #define FAIL( S, ... ) do { fprintf( stderr, "mia_gpu_mg: " __VA_ARGS__ ); (S)->failed = 1; } while ( 0 )
@@ -272,6 +287,16 @@ static void* worker( void* arg_ ) {
     SYNC( S );
     if ( S->converged || S->iter >= MAX_ITER ) break;
   }
+  if ( S->damage_fn ) {                                             /* the contexts still hold the final round: the ranks' tables, summed */
+    CK( S, miagpu_misincorporation( g, S->damage[rank] ) );
+    SYNC( S );
+    if ( rank == 0 ) {
+      int r, c;
+      for ( r = 1; r < world; r++ )
+        for ( c = 0; c < MIAGPU_MISINC_INTS; c++ ) S->damage[0][c] += S->damage[r][c];
+      if ( !write_damage( S->damage_fn, S->damage[0] ) ) FAIL( S, "cannot write %s\n", S->damage_fn );
+    }
+  }
   miagpu_destroy( g );
   return NULL;
 }
@@ -288,6 +313,10 @@ int main( int argc, char** argv ) {
     else if ( !strcmp( argv[i], "-F" ) ) S.final_only = 1;
     else if ( !strcmp( argv[i], "-h" ) ) S.hp_special = 1;
     else if ( !strcmp( argv[i], "-i" ) ) ;
+    else if ( !strcmp( argv[i], "-d" ) ) {
+      if ( i + 1 >= argc ) { fprintf( stderr, "mia_gpu_mg: -d needs a file name (the damage profile of the final round)\n" ); return 2; }
+      S.damage_fn = argv[++i];
+    }
     else if ( i + 1 < argc && !strcmp( argv[i], "-g" ) ) ngpu = atoi( argv[++i] );
     else if ( i + 1 < argc && !strcmp( argv[i], "-r" ) ) ref_fn = argv[++i];
     else if ( i + 1 < argc && !strcmp( argv[i], "-f" ) ) frag_fn = argv[++i];
@@ -301,7 +330,8 @@ int main( int argc, char** argv ) {
     else { fprintf( stderr, "mia_gpu_mg: option %s is not handled by this host (see the header of host/mia_gpu_mg.c)\n", argv[i] ); return 2; }
   }
   if ( !ref_fn || !frag_fn || !mat_fn ) {
-    fprintf( stderr, "usage: mia_gpu_mg -g N -r ref.fa -f reads.fa|fq -s matrix.txt [-m root] [-c] [-k K] [-p code] [-H cut | -S slope -N icpt] [-F]\n" );
+    fprintf( stderr, "usage: mia_gpu_mg -g N -r ref.fa -f reads.fa|fq -s matrix.txt [-m root] [-c] [-k K] [-p code] [-H cut | -S slope -N icpt] [-F]\n"
+                     "                  [-d damage.tsv  (extension of this host: the final round's misincorporation table)]\n" );
     return 2;
   }
   init_comp();

@@ -561,6 +561,25 @@ int miagpu_write_maln( const char* path, const miagpu_maln_header* hd,
 int miagpu_write_maln_fsdb( miagpu_ctx* ctx, const char* path, const miagpu_maln_header* hd,
                             const miagpu_maln_reads* rd, int64_t* n_alnseqs_out );
 
+/* ---- Damage profile of the last round: the misincorporation table of its culled alignments, computed on the device from the
+ * entry list the consensus walked (no `.maln` file needed).  counts[d][r][q], int64 [31][6][6], r (reference) and q (read) over
+ * A C G T N - (N = any other character), summed over every AlnSeq of the round's `.maln` with DR 0:
+ *   aligned columns  every column c of SEQ with START + c < LEN: d = SMP[c] - 'A', r = the reference's SEQ at START + c,
+ *                    q = SEQ[c] ('-': the read has a deletion there)
+ *   inserted bases   every base of INS_POS in front of such a column c: r = '-', q = the inserted base, d = SMP[c]
+ *   orientation      an AlnSeq with RC 1 has both bases complemented (A<->T, C<->G; N and - stay) and d -> 30 - d, so depth 0
+ *                    is always the molecule's 5' end and every cell is the cell of the FORWARD matrix (miagpu_set_pssm) that
+ *                    scored the base (revcom_pssm: rev[30-d][i][j] = fwd[d][comp i][comp j]).
+ * Records that stale pointers reach and frozen slot content count as the file lists them; dropped AlnSeqs and reads that are not
+ * unique_best (-u / -U) count nowhere.  Integer sums: the same for any schedule; the table of a sharded round is the sum of the
+ * ranks' tables.  Valid after a call that ends a round with base calling on this context (miagpu_iterate_resident,
+ * miagpu_iterate_host, miagpu_consensus, miagpu_consensus_natural, miagpu_shard_finish); a later call that changes the reference,
+ * the reads, their strands, their alignments or the entry list (miagpu_set_reference, miagpu_upload_reads, miagpu_compact_reads,
+ * miagpu_set_alignment_inputs, the realign / pass-1 / window calls, miagpu_accumulate_gaps*, miagpu_set_fsdb,
+ * miagpu_distant_retry*, miagpu_shard_begin*) makes the call fail with a miagpu_last_error that says which.  Changes no state the next round reads. */
+#define MIAGPU_MISINC_INTS 1116       /* 31 depths x 6 reference codes x 6 read codes */
+int miagpu_misincorporation( miagpu_ctx* ctx, int64_t* counts );
+
 /* ---- measurement helpers (bench.py) */
 /* per width bucket of the last realign: columns-per-lane K (0 = too wide),
  * reads, DP cells, kernel ms (CUDA events on the library's stream); MIAGPU_NBUCKET entries */

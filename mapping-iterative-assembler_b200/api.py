@@ -12,6 +12,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MIAGPU_LIB") or os.path.join(HERE, "libmiagpu.so")      # MIAGPU_LIB: a differently built libmiagpu.so (kernel experiments)
 MAX_RUNS = 24
 RUN_M, RUN_I, RUN_D = 0, 1, 2
+MISINC_SHAPE = (31, 6, 6)          # miagpu_misincorporation: depth, reference, read
+MISINC_CODES = "ACGTN-"            # the codes of both base axes (N = any other character)
 
 _i32p = C.POINTER(C.c_int32)
 _u8p = C.POINTER(C.c_uint8)
@@ -110,6 +112,7 @@ def load_library():
     L.miagpu_distant_retry.argtypes = [C.c_void_p, _i64p, _i64p]
     L.miagpu_distant_retry_begin.argtypes = [C.c_void_p, _i64p, _i32p]
     L.miagpu_distant_retry_end.argtypes = [C.c_void_p, C.c_int, _i64p]
+    L.miagpu_misincorporation.argtypes = [C.c_void_p, _i64p]
     L.miagpu_stream.restype = C.c_void_p
     L.miagpu_stream.argtypes = [C.c_void_p]
     _lib = L
@@ -127,7 +130,7 @@ EXPORTS = ["miagpu_device_count", "miagpu_create", "miagpu_destroy", "miagpu_las
            "miagpu_fastx_open", "miagpu_fastx_open_memory", "miagpu_fastx_format", "miagpu_fastx_next", "miagpu_fastx_batch", "miagpu_fastx_close",
            "miagpu_maln_ref_size", "miagpu_write_maln", "miagpu_read_pssm", "miagpu_align_windows",
            "miagpu_set_fsdb", "miagpu_get_fsdb", "miagpu_last_fsdb_stats", "miagpu_distant_retry", "miagpu_write_maln_fsdb", "miagpu_last_pass1_cells", "miagpu_set_homopolymer", "miagpu_shard_flags", "miagpu_set_cons_capacity",
-           "miagpu_distant_retry_begin", "miagpu_distant_retry_end"]
+           "miagpu_distant_retry_begin", "miagpu_distant_retry_end", "miagpu_misincorporation"]
 
 
 def _ptr(a):
@@ -342,6 +345,13 @@ class MiaGpu:
         b = C.c_int64()
         self._ck(self.lib.miagpu_distant_retry_end(self.h, int(state_in), C.byref(b)))
         return b.value
+
+    def misincorporation(self):
+        """Damage profile of the last round (miagpu_misincorporation): int64[31, 6, 6] = counts[depth][reference][read] over
+        MISINC_CODES, in the orientation of the molecule (depth 0 = its 5' end), cell for cell the forward matrix's."""
+        t = np.zeros(MISINC_SHAPE, np.int64)
+        self._ck(self.lib.miagpu_misincorporation(self.h, t.ctypes.data_as(_i64p)))
+        return t
 
     def reset_dropped(self):
         self._ck(self.lib.miagpu_reset_dropped(self.h))

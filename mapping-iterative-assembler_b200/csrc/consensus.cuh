@@ -108,12 +108,43 @@ __device__ __forceinline__ void add_base_dev(const Adder& A, Col col, int ch_cod
   for (int x = 0; x < 4; x++) A.add(PL_SCORE + x, col, m[x * 5]);
 }
 
+// Misincorporation table (miagpu_misincorporation): counts[depth][ref][read] over A C G T N -, in the orientation of the molecule
+// (a reverse-strand entry is complemented and mirrored, depth -> 30 - depth, so every cell is the cell of the FORWARD matrix that
+// scored the base).  The bins are skewed: with 35-75 bp reads about half of all columns are matches at depth 15, where the 32
+// lanes of a warp would hit four shared addresses.  Those four cells are lane-private register counters, summed over the warp
+// once per block; everything else (the depths of the read ends, where consecutive lanes have consecutive depths, mismatches,
+// deletions, inserted bases) is a shared-memory atomic into the block's table.
+constexpr int MISINC_CODES = 6;                 // A C G T N -
+struct MisincAdder {
+  uint32_t* s_tab;                              // [31][6][6] of this block
+  const uint8_t* ref;                           // reference codes 0..4
+  mutable uint32_t hot0 = 0, hot1 = 0, hot2 = 0, hot3 = 0;   // depth-15 matches of this lane, by forward base
+  __device__ __forceinline__ static int comp(int b) { return b < 4 ? 3 - b : b; }
+  // an aligned column: reference position pos, read code qc (5 = the read has a deletion)
+  __device__ __forceinline__ void base(int depth, int pos, int qc, bool rev) const {
+    int r = ref[pos];
+    if (rev) { r = comp(r); qc = comp(qc); depth = 2 * PSSM_DEPTH - depth; }
+    if (depth == PSSM_DEPTH && r == qc && r < 4) {
+      hot0 += r == 0; hot1 += r == 1; hot2 += r == 2; hot3 += r == 3;
+    } else {
+      atomicAdd(s_tab + (depth * MISINC_CODES + r) * MISINC_CODES + qc, 1u);
+    }
+  }
+  // an inserted base in front of a column of depth `depth`: reference '-'
+  __device__ __forceinline__ void ins(int depth, int qc, bool rev) const {
+    if (rev) { qc = comp(qc); depth = 2 * PSSM_DEPTH - depth; }
+    atomicAdd(s_tab + (depth * MISINC_CODES + 5) * MISINC_CODES + qc, 1u);
+  }
+};
+
 // One entry, walked by a whole warp (lanes take consecutive reference columns).
 // MODE 0: ref->gaps = max insert length per position over the culled list (mia.c:486-504;
 //         positions with start < pos <= end only, so an insert in front of an entry's first
 //         column never counts)
 // MODE 1: base columns + insert columns
 // MODE 2: base columns only (what AlnSeq.dropped decides, mia.c:571-579; insert columns count dropped reads too)
+// MODE 3: the misincorporation table (MisincAdder): every column below seq_len and every inserted base in front of one, of the
+//         entries that are not dropped -- what the AlnSeq's SEQ / INS_POS / SMP in the `.maln` file list
 // Where the columns of a reference position lie.  GlobalLay: the padded layout of the whole alignment, straight from ins_off / gaps.
 // TileLay: the same for an entry that lies wholly inside a tile's shared window -- columns relative to the window, insert offsets
 // and lengths from the tile's copy of ins_off (gaps[pos] = ins_off[pos + 1] - ins_off[pos] for pos > 0, the only positions asked).
@@ -134,7 +165,7 @@ struct TileLay {
 
 template <int MODE, typename Adder, typename Lay>
 __device__ __forceinline__ void walk_entry(const ConsParams& p, const miagpu_entry& e, int lane, const Adder& A, const Lay& Y, const int32_t* sm) {
-  if (e.col_count <= 0) return;
+  if (e.col_count <= 0 || (MODE == 3 && e.dropped)) return;
   const int rd = e.read;
   const bool fz = rd >= p.n_reads;
   const int64_t q = rd - p.n_reads;
@@ -142,7 +173,8 @@ __device__ __forceinline__ void walk_entry(const ConsParams& p, const miagpu_ent
   if (nr <= 0) return;
   const uint16_t* runs = fz ? p.fz_runs + q * MAX_RUNS : p.runs + (int64_t)rd * MAX_RUNS;
   const uint8_t* read = fz ? p.fz_bases + q * FZ_BASES_STRIDE : p.bases + p.off[rd];
-  const int32_t* sm_strand = sm + ((fz ? p.fz_rc[q] : p.rc[rd]) ? MIAGPU_PSSM_INTS : 0);
+  const bool rev = fz ? p.fz_rc[q] : p.rc[rd];
+  const int32_t* sm_strand = sm + (rev ? MIAGPU_PSSM_INTS : 0);
   const int cb = e.col_begin, ce = e.col_begin + e.col_count;
 
   int colpos = 0;                 // reference columns before this run
@@ -162,6 +194,10 @@ __device__ __forceinline__ void walk_entry(const ConsParams& p, const miagpu_ent
       const int q = (i == colpos) ? pend : 0;               // insert length in front of this column
       if (MODE == 0) {
         if (q > 0 && i > cb && pos > 0) atomicMax(p.gaps + pos, q);
+      } else if constexpr (MODE == 3) {
+        const int depth = smp_depth(e, e.act_bias + (isM ? row - row0 : rpos - row0));
+        A.base(depth, pos, isM ? base_code(read[row]) : 5, rev);
+        for (int j = 0; j < q; j++) A.ins(depth, base_code(read[row - q + j]), rev);   // INS_POS: every insert, first column too
       } else {
         // act = read bases consumed before the column, inserted ones included (fsdb.c:564-583)
         const int act = e.act_bias + (isM ? row - row0 : rpos - row0);
@@ -370,6 +406,49 @@ __global__ void __launch_bounds__(256) undo_kernel(ConsParams p, int64_t n_reads
       if (lane == 0) entries[idx].dropped = 1;
     }
   }
+}
+
+// The misincorporation table of the entry list (MODE 3 of walk_entry), read only: a block takes MISINC_PER_BLOCK consecutive
+// entries (at most 2 M columns: the block-private 32-bit cells cannot overflow) and adds its table into the global 64-bit one once.
+// A warp takes 32 entries at a time; each lane first touches the per-read words and the bases of its entry, so that 32 of those
+// dependent loads are in flight at once before the warp walks the 32 entries one by one (DESIGN 4.12: the walk is latency-bound).
+constexpr int MISINC_THREADS = 256;
+constexpr int MISINC_PER_BLOCK = 4096;
+__global__ void __launch_bounds__(MISINC_THREADS) misinc_kernel(ConsParams p, const uint8_t* __restrict__ ref, unsigned long long* out) {
+  __shared__ uint32_t s_tab[MIAGPU_MISINC_INTS];
+  for (int i = threadIdx.x; i < MIAGPU_MISINC_INTS; i += blockDim.x) s_tab[i] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  const MisincAdder A{s_tab, ref};
+  const int64_t b0 = (int64_t)blockIdx.x * MISINC_PER_BLOCK, b1 = min(b0 + MISINC_PER_BLOCK, p.n_entries);
+  for (int64_t base = b0 + warp * 32; base < b1; base += nwarps * 32) {
+    if (base + lane < b1) {
+      const int rd = p.entries[base + lane].read;
+      if (rd < p.n_reads) {
+        asm volatile("prefetch.global.L1 [%0];" ::"l"(p.n_runs + rd));
+        asm volatile("prefetch.global.L1 [%0];" ::"l"(p.abr + rd));
+        asm volatile("prefetch.global.L1 [%0];" ::"l"(p.rc + rd));
+        asm volatile("prefetch.global.L1 [%0];" ::"l"(p.runs + (int64_t)rd * MAX_RUNS));
+        const int64_t o0 = p.off[rd], o1 = p.off[rd + 1];
+        if (o1 > o0) {
+          asm volatile("prefetch.global.L1 [%0];" ::"l"(p.bases + o0));
+          asm volatile("prefetch.global.L1 [%0];" ::"l"(p.bases + o1 - 1));
+        }
+      }
+    }
+    const int m = (int)min((int64_t)32, b1 - base);
+    for (int k = 0; k < m; k++) walk_entry<3>(p, load_entry(p.entries + base + k), lane, A);
+  }
+  uint32_t h[4] = {A.hot0, A.hot1, A.hot2, A.hot3};
+#pragma unroll
+  for (int r = 0; r < 4; r++) {
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) h[r] += __shfl_xor_sync(0xffffffffu, h[r], s);
+    if (lane == 0 && h[r]) atomicAdd(s_tab + (PSSM_DEPTH * MISINC_CODES + r) * MISINC_CODES + r, h[r]);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < MIAGPU_MISINC_INTS; i += blockDim.x)
+    if (s_tab[i]) atomicAdd(out + i, (unsigned long long)s_tab[i]);
 }
 
 // Entries binned by the tile their first column lies in (a counting sort in two kernels; the order inside a bin does not

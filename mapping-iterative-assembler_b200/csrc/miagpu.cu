@@ -232,12 +232,23 @@ struct miagpu_ctx {
   std::vector<FsExtra> fs_extra;               // this round's stale pointers, in FSDB order (front before back)
   std::vector<int32_t> fs_patch_host;          // smp parameters the writer needs for slots whose last visitor is a stale pointer
   miagpu_ctx* aux = nullptr;                   // scratch context of the -D attempts
+  // miagpu_misincorporation: whether the entry list, alignments, reads and reference on the device are still those of the last
+  // round that ended with base calling, and if not, the call that changed them
+  const char* misinc_stale = "no round has ended with base calling on this context";
+  DevBuf<unsigned long long> d_misinc;
+  cudaEvent_t misinc_ev[3] = {};               // its own timing events: the rounds' events may still be read between their calls
   // timing of the last call
   float ms_kernels = 0, ms_h2d = 0, ms_d2h = 0;
   int64_t dp_cells = 0;
   int launches = 0;
 };
 
+
+// the table of miagpu_misincorporation belongs to the state the last round left: the first call after it that changes that state
+// is what a refusal names (before any round: that there was none)
+static void misinc_invalidate(miagpu_ctx* c, const char* why) {
+  if (!c->misinc_stale) c->misinc_stale = why;
+}
 
 // -------------------------------------------------------------------- misc
 extern "C" const char* miagpu_last_error(void) { return g_err; }
@@ -333,7 +344,8 @@ extern "C" void miagpu_destroy(miagpu_ctx* c) {
   c->d_back_slot.release(); c->d_first.release(); c->d_nsl.release(); c->d_slot_owner.release(); c->d_slot_owner_prev.release();
   c->d_ent_slot.release(); c->d_stale.release(); c->d_fs_cnt.release(); c->d_fs_tmp.release(); c->d_nprefix.release();
   c->d_runs_prev.release(); c->d_nruns_prev.release(); c->d_abr_prev.release(); c->d_as_prev.release(); c->d_ae_prev.release(); c->d_score_prev.release();
-  c->d_fz_bases.release(); c->d_fz_rc.release(); c->d_fz_runs.release(); c->d_fz_nruns.release();
+  c->d_fz_bases.release(); c->d_fz_rc.release(); c->d_fz_runs.release(); c->d_fz_nruns.release(); c->d_misinc.release();
+  for (auto& ev : c->misinc_ev) if (ev) cudaEventDestroy(ev);
   if (c->aux) miagpu_destroy(c->aux);
   cudaStreamDestroy(c->stream);
   delete c;
@@ -422,6 +434,7 @@ static int upload_codes(miagpu_ctx* c, const std::string& s, DevBuf<uint8_t>& ds
 
 extern "C" int miagpu_set_reference(miagpu_ctx* c, const char* seq, int seq_len, int circular, int with_rc) {
   if (!c || !seq || seq_len <= 0) { set_error("miagpu_set_reference: bad argument"); return 0; }
+  misinc_invalidate(c, "miagpu_set_reference has replaced the reference of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   int wrap = circular ? std::min(seq_len, MAX_READ) : 0;         // add_ref_wrap, mia.c:657-689
   c->seq_len = seq_len;
@@ -499,6 +512,7 @@ static int reserve_per_read(miagpu_ctx* c, int64_t n) {
 
 extern "C" int miagpu_upload_reads(miagpu_ctx* c, int64_t n, const uint8_t* bases, const int64_t* offsets) {
   if (!c || n < 0 || (n > 0 && (!bases || !offsets))) { set_error("miagpu_upload_reads: bad argument"); return 0; }
+  misinc_invalidate(c, "miagpu_upload_reads has replaced the reads of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   if (n > 0x7fffffffLL / NBUCKET) { set_error("miagpu_upload_reads: at most %lld reads per batch", 0x7fffffffLL / NBUCKET); return 0; }
   int64_t total = n ? offsets[n] : 0;
@@ -1144,6 +1158,7 @@ static int realign_common(miagpu_ctx* c, const uint8_t* rc, const int32_t* as, c
                           int32_t* as_out, int32_t* ae_out, int32_t* abr, int32_t* n_runs, uint16_t* runs, uint8_t* status,
                           bool time_h2d_from_upload) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("miagpu_realign: set_pssm and set_reference first"); return 0; }
+  misinc_invalidate(c, "a realign has replaced the alignments of that round");
   if (c->n && (!rc || !as || !ae)) { set_error("miagpu_realign: rc/as/ae are required"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   const int64_t n = c->n;
@@ -1194,6 +1209,7 @@ extern "C" int miagpu_align_windows(miagpu_ctx* c, const uint8_t* rc, const int3
                                     int32_t* score, int32_t* as_out, int32_t* ae_out, int32_t* abr, int32_t* n_runs, uint16_t* runs,
                                     uint8_t* status) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("miagpu_align_windows: set_pssm and set_reference first"); return 0; }
+  misinc_invalidate(c, "miagpu_align_windows has replaced the alignments of that round");
   const int64_t n = c->n;
   if (n && (!rc || !win_start || !win_len)) { set_error("miagpu_align_windows: rc / win_start / win_len are required"); return 0; }
   std::vector<int32_t> win_end((size_t)n);
@@ -1251,6 +1267,7 @@ extern "C" int miagpu_last_pair_buckets(miagpu_ctx* c, int32_t* k, int32_t* read
 // nothing crosses PCIe except the consensus string.
 extern "C" int miagpu_set_alignment_inputs(miagpu_ctx* c, const uint8_t* rc, const int32_t* as, const int32_t* ae) {
   if (!c || (c->n && (!rc || !as || !ae))) { set_error("miagpu_set_alignment_inputs: bad argument"); return 0; }
+  misinc_invalidate(c, "miagpu_set_alignment_inputs has replaced the strands of that round's reads");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   if (c->n) {
     MIAGPU_CUDA(cudaMemcpyAsync(c->d_rc.p, rc, c->n, cudaMemcpyHostToDevice, c->stream));
@@ -1299,6 +1316,7 @@ extern "C" int miagpu_get_alignment(miagpu_ctx* c, int32_t* score, int32_t* as_o
 
 extern "C" int miagpu_realign_resident(miagpu_ctx* c) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("miagpu_realign_resident: set_pssm and set_reference first"); return 0; }
+  misinc_invalidate(c, "miagpu_realign_resident has replaced the alignments of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   MIAGPU_CUDA(cudaEventRecord(c->ev[1], c->stream));
   if (!realign_device(c)) return 0;
@@ -1469,6 +1487,7 @@ static int launch_accumulate(miagpu_ctx* c) {
 
 extern "C" int miagpu_accumulate_gaps(miagpu_ctx* c, int64_t n_entries, const miagpu_entry* entries, void** dev_gaps, int64_t* n_gaps) {
   if (!c || !c->have_ref || !c->have_pssm) { set_error("miagpu_accumulate_gaps: set_pssm / set_reference / realign first"); return 0; }
+  misinc_invalidate(c, "miagpu_accumulate_gaps has replaced the entry list of that round");
   if (n_entries < 0 || (n_entries && !entries)) { set_error("miagpu_accumulate_gaps: bad entries"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   for (int64_t i = 0; i < n_entries; i++) {
@@ -1592,6 +1611,7 @@ extern "C" int miagpu_set_cons_capacity(miagpu_ctx* c, int64_t bytes) {
 extern "C" int miagpu_accumulate_gaps_natural(miagpu_ctx* c, const uint8_t* dropped_front, const uint8_t* dropped_back,
                                               void** dev_gaps, int64_t* n_gaps) {
   if (!c || !c->have_ref || !c->have_pssm) { set_error("miagpu_accumulate_gaps_natural: set_pssm / set_reference / realign first"); return 0; }
+  misinc_invalidate(c, "miagpu_accumulate_gaps_natural has replaced the entry list of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   const int64_t n = c->n;
   c->launches = 0;
@@ -1629,6 +1649,7 @@ extern "C" int miagpu_consensus_natural(miagpu_ctx* c, const uint8_t* dropped_fr
   if (!miagpu_accumulate_counts(c, nullptr, nullptr)) return 0;
   if (!miagpu_call(c, cons_code, gaps_out, counts_out, cons_out, cons_len)) return 0;
   c->ms_h2d = h2d;
+  c->misinc_stale = nullptr;
   return 1;
 }
 
@@ -1760,6 +1781,33 @@ extern "C" int miagpu_consensus(miagpu_ctx* c, int64_t n_entries, const miagpu_e
   if (!miagpu_accumulate_counts(c, nullptr, nullptr)) return 0;
   if (!miagpu_call(c, cons_code, gaps_out, counts_out, cons_out, cons_len)) return 0;
   c->ms_h2d = h2d;
+  c->misinc_stale = nullptr;
+  return 1;
+}
+
+// ---- damage profile: the misincorporation table of the entry list the last round's consensus walked (misinc_kernel, MODE 3 of
+// walk_entry).  Reads the entries, alignments, reads and reference as the round left them and writes only its own buffer.
+extern "C" int miagpu_misincorporation(miagpu_ctx* c, int64_t* counts) {
+  if (!c || !counts) { set_error("miagpu_misincorporation: NULL argument"); return 0; }
+  if (c->misinc_stale) { set_error("miagpu_misincorporation: no table of the last round: %s", c->misinc_stale); return 0; }
+  MIAGPU_CUDA(cudaSetDevice(c->device));
+  for (auto& ev : c->misinc_ev) if (!ev) MIAGPU_CUDA(cudaEventCreate(&ev));
+  if (!c->d_misinc.reserve(MIAGPU_MISINC_INTS)) return 0;
+  MIAGPU_CUDA(cudaEventRecord(c->misinc_ev[0], c->stream));
+  MIAGPU_CUDA(cudaMemsetAsync(c->d_misinc.p, 0, MIAGPU_MISINC_INTS * sizeof(unsigned long long), c->stream));
+  if (c->n_entries) {
+    misinc_kernel<<<(unsigned)((c->n_entries + MISINC_PER_BLOCK - 1) / MISINC_PER_BLOCK), MISINC_THREADS, 0, c->stream>>>(cons_params(c), c->d_ref.p,
+                                                                                                                       c->d_misinc.p);
+    MIAGPU_CUDA(cudaGetLastError());
+  }
+  MIAGPU_CUDA(cudaEventRecord(c->misinc_ev[1], c->stream));
+  MIAGPU_CUDA(cudaMemcpyAsync(counts, c->d_misinc.p, MIAGPU_MISINC_INTS * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  MIAGPU_CUDA(cudaEventRecord(c->misinc_ev[2], c->stream));
+  MIAGPU_CUDA(cudaStreamSynchronize(c->stream));
+  MIAGPU_CUDA(cudaEventElapsedTime(&c->ms_kernels, c->misinc_ev[0], c->misinc_ev[1]));
+  MIAGPU_CUDA(cudaEventElapsedTime(&c->ms_d2h, c->misinc_ev[1], c->misinc_ev[2]));
+  c->ms_h2d = 0;
+  c->launches = c->n_entries ? 1 : 0;
   return 1;
 }
 
@@ -2110,6 +2158,7 @@ extern "C" int miagpu_set_fsdb(miagpu_ctx* c, const int32_t* seq_len, const uint
                                const uint8_t* strand_known, const int32_t* front_slot, const int32_t* back_slot, int64_t n_slots,
                                const uint8_t* slot_dropped, int distant_ref) {
   if (!c || (c->n && (!seq_len || !score))) { set_error("miagpu_set_fsdb: seq_len and score are required"); return 0; }
+  misinc_invalidate(c, "miagpu_set_fsdb has replaced the pointer state of that round");
   if ((front_slot == nullptr) != (back_slot == nullptr) || n_slots < 0) { set_error("miagpu_set_fsdb: front_slot and back_slot come together"); return 0; }
   if (!miagpu_set_cut_inputs(c, seq_len, unique_best, nullptr)) return 0;
   const int64_t n = c->n;
@@ -2238,6 +2287,7 @@ static int distant_chain(miagpu_ctx* c, int state_in, bool apply, std::vector<in
 extern "C" int miagpu_distant_retry_begin(miagpu_ctx* c, int64_t* n_tried, int32_t* state_after) {
   if (n_tried) *n_tried = 0;
   if (!c || !c->fs_on || !c->have_ref || !c->have_pssm) { set_error("miagpu_distant_retry: set_pssm, set_reference and miagpu_set_fsdb first"); return 0; }
+  misinc_invalidate(c, "miagpu_distant_retry has realigned reads of that round");
   c->dr_U.clear(); c->dr_sc.clear(); c->dr_a0.clear(); c->dr_a1.clear(); c->dr_score.clear();
   c->dr_ready = true;
   if (!c->fs_distant) { if (state_after) { state_after[0] = 0; state_after[1] = 1; } return 1; }
@@ -2291,6 +2341,7 @@ extern "C" int miagpu_distant_retry_begin(miagpu_ctx* c, int64_t* n_tried, int32
 extern "C" int miagpu_distant_retry_end(miagpu_ctx* c, int state_in, int64_t* n_learned) {
   if (n_learned) *n_learned = 0;
   if (!c || !c->fs_on || !c->dr_ready) { set_error("miagpu_distant_retry_end: call miagpu_distant_retry_begin first"); return 0; }
+  misinc_invalidate(c, "miagpu_distant_retry_end has realigned reads of that round");
   c->dr_ready = false;
   if (state_in != 0 && state_in != 1) { set_error("miagpu_distant_retry_end: state_in is 0 (forward matrix) or 1 (strand-reversed)"); return 0; }
   if (c->dr_U.empty()) return 1;
@@ -2319,6 +2370,7 @@ extern "C" int miagpu_distant_retry(miagpu_ctx* c, int64_t* n_tried, int64_t* n_
   if (n_tried) *n_tried = 0;
   if (n_learned) *n_learned = 0;
   if (!c || !c->fs_on || !c->have_ref || !c->have_pssm) { set_error("miagpu_distant_retry: set_pssm, set_reference and miagpu_set_fsdb first"); return 0; }
+  misinc_invalidate(c, "miagpu_distant_retry has realigned reads of that round");
   if (!c->fs_distant || c->fs_round < 1) return 1;   // iter_num > 1 only (mia_main.c:122)
   return miagpu_distant_retry_begin(c, n_tried, nullptr) && miagpu_distant_retry_end(c, c->fs_submat_rc, n_learned);
 }
@@ -2570,6 +2622,7 @@ static int host_round_front(miagpu_ctx* c, const char* who, int64_t n, const uin
                             int32_t* n_runs, uint8_t* status, const int32_t* seq_len, const uint8_t* unique_best, bool stats,
                             const uint8_t* dropped, const Trace& tr, int* chunks) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("%s: set_pssm and set_reference first", who); return 0; }
+  misinc_invalidate(c, "a new round has started and not ended");
   if (n <= 0 || !bases || !offsets || !rc || !as || !ae || !score || !seq_len || !dropped) { set_error("%s: bad argument", who); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   if (n > 0x7fffffffLL / NBUCKET) { set_error("%s: at most %lld reads per batch", who, 0x7fffffffLL / NBUCKET); return 0; }
@@ -2677,7 +2730,9 @@ extern "C" int miagpu_iterate_host(miagpu_ctx* c, int64_t n, const uint8_t* base
     float ms = 0;
     if (cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]) == cudaSuccess) fprintf(stderr, "[miagpu trace] DP of %d chunk(s) on the device: %.3f ms\n", C, ms);
   }
-  return host_round_stats(c, C);
+  if (!host_round_stats(c, C)) return 0;
+  c->misinc_stale = nullptr;
+  return 1;
 }
 
 // The same round over reads, rc/as/ae, seq_len / unique_best and sticky flags that are already resident:
@@ -2711,6 +2766,7 @@ extern "C" int miagpu_iterate_resident(miagpu_ctx* c, int hard_cut, int score_cu
                                        double* slope_out, double* intercept_out, uint8_t* dropped, int32_t* gaps_out, char* cons_out,
                                        int32_t* cons_len) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("miagpu_iterate_resident: set_pssm and set_reference first"); return 0; }
+  misinc_invalidate(c, "a new round has started and not ended");
   if (c->n <= 0 || c->cut_inputs_n != c->n) { set_error("miagpu_iterate_resident: upload reads, alignment inputs and cut inputs first"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   const int64_t n = c->n;
@@ -2756,6 +2812,7 @@ extern "C" int miagpu_iterate_resident(miagpu_ctx* c, int hard_cut, int score_cu
     c->fs_prev_seq_len = c->seq_len;                 // the geometry of this round's alignments, should the next round have to freeze one
     fs_carry_submat(c);
   }
+  c->misinc_stale = nullptr;
   return 1;
 }
 
@@ -2836,6 +2893,7 @@ static int shard_after_dp(miagpu_ctx* c, bool stats_done, bool has_unique, void*
 
 static int shard_args(miagpu_ctx* c, const char* who, int world, int rank, int64_t n_max, int64_t n) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("%s: set_pssm and set_reference first", who); return 0; }
+  misinc_invalidate(c, "a new round has started and not ended");
   if (world < 1 || rank < 0 || rank >= world || n_max < n || n_max < 1) { set_error("%s: bad world / rank / n_max (n_max must be the largest read count of any rank)", who); return 0; }
   if ((int64_t)world * (n_max + CUT_BLOCK) > 0x7fffffffLL * 64) { set_error("%s: too many reads", who); return 0; }
   return 1;
@@ -3094,12 +3152,15 @@ extern "C" int miagpu_shard_finish(miagpu_ctx* c, int cons_code, uint8_t* droppe
   MIAGPU_CUDA(cudaStreamSynchronize(down));
   if (c->sh_host) {
     MIAGPU_CUDA(cudaStreamSynchronize(c->s_up));
-    return host_round_stats(c, c->sh_chunks);
+    if (!host_round_stats(c, c->sh_chunks)) return 0;
+    c->misinc_stale = nullptr;
+    return 1;
   }
   c->ms_kernels = ms_dp;
   c->ms_h2d = c->ms_d2h = 0;
   MIAGPU_CUDA(cudaMemcpy(&c->n_fallback, c->d_meta.p + META_NFALL, 4, cudaMemcpyDeviceToHost));
   if (c->fs_on) c->fs_prev_seq_len = c->seq_len;     // the geometry of this round's alignments, should the next round have to freeze one
+  c->misinc_stale = nullptr;
   return 1;
 }
 
@@ -3674,6 +3735,7 @@ static int pass1_sweep(miagpu_ctx* c, const PairLmax& lm) {
 extern "C" int miagpu_pass1(miagpu_ctx* c, int32_t* hits, int32_t* score, int32_t* fw_score, int32_t* rc_score, uint8_t* rc, int32_t* as,
                             int32_t* ae, int32_t* start, int32_t* end, int32_t* abr, int32_t* n_runs, uint16_t* runs, uint8_t* status) {
   if (!c || !c->have_pssm || !c->have_ref || !c->with_rc) { set_error("miagpu_pass1: set_pssm and set_reference(with_rc=1) first"); return 0; }
+  misinc_invalidate(c, "miagpu_pass1 has replaced the alignments of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   const int64_t n = c->n;
   c->launches = 0;
@@ -3771,6 +3833,7 @@ __global__ void compact_kernel(int64_t n_new, const int32_t* src, const uint8_t*
 
 extern "C" int miagpu_compact_reads(miagpu_ctx* c, const uint8_t* keep, const uint8_t* revcomp, int64_t* n_out) {
   if (!c || (c->n && !keep)) { set_error("miagpu_compact_reads: bad argument"); return 0; }
+  misinc_invalidate(c, "miagpu_compact_reads has replaced the reads of that round");
   MIAGPU_CUDA(cudaSetDevice(c->device));
   std::vector<int64_t> off_old(c->n + 1), off_new(1, 0);
   if (c->n) MIAGPU_CUDA(cudaMemcpy(off_old.data(), c->d_off.p, (c->n + 1) * 8, cudaMemcpyDeviceToHost));

@@ -384,6 +384,14 @@ class ResidentAssembler:
         self.cons = cons
         return cons, cons == self.last
 
+    def misincorporation(self):
+        """Damage profile of the last round: int64[31, 6, 6] (api.MiaGpu.misincorporation); with an `exchange`, the sum over the
+        ranks -- the table of the whole round, the same as one GPU's."""
+        t = self.g.misincorporation()
+        if self.x is None:
+            return t
+        return self._gather(t.ravel()).reshape((-1,) + api.MISINC_SHAPE).sum(0)
+
     def write_maln(self, path, batch, ref_id, ref_desc=""):
         """write_ma of this round's culled_maln (mia_main.c:905 / 958) from the device's results: `batch` is the FastxReader batch
         (or any dict with bases / offsets / ids / id_off / descs / desc_off) the reads came from, in input order; call after
