@@ -441,7 +441,8 @@ int miagpu_adopt_alignment( miagpu_ctx* ctx, int32_t* score, int32_t* as, int32_
  * pop_s2c_in_a, dyn_prog, max_sg_score, find_align_begin, populate_pwaln_to_begin) and that reiterate_assembly runs after
  * its window rule: every resident read against its own stretch [win_start, win_start + win_len) of the resident reference
  * (for ccheck: the lifted-over consensus pieces back to back, set with miagpu_set_reference( circular = 0 ); matrix =
- * init_flatsubmat through miagpu_set_pssm), unmasked, sg5 as given, rc[i] picks the strand-reversed matrix.  No window rule,
+ * init_flatsubmat through miagpu_set_pssm), unmasked, sg5 as given at every window width (windows over 512 columns go to the
+ * chunked kernel, which takes sg5 too; homopolymer mode refuses sg5 = 0), rc[i] picks the strand-reversed matrix.  No window rule,
  * no fall-back to the whole reference; a window may be shorter than its read.  Outputs as miagpu_realign (as_out / ae_out are
  * reference coordinates: abc + win_start, aec + win_start).  Overwrites the resident as / ae of
  * miagpu_set_alignment_inputs. */

@@ -772,7 +772,8 @@ static int launch_strip(miagpu_ctx* c, int mode, const int32_t* list, int n_list
   p.list = list; p.n_list = n_list; p.n_list_ptr = n_list_ptr; p.rc_in = c->d_rc.p;
   p.ref_codes[0] = c->d_ref.p; p.ref_codes[1] = c->with_rc ? c->d_rcref.p : c->d_ref.p;
   p.len1 = len1; p.seq_len = c->seq_len; p.prof = c->d_prof.p;
-  p.k = mode == 0 ? c->kmer_k : 0;
+  p.sg5 = c->explicit_windows ? c->explicit_sg5 : 1;            // miagpu_align_windows' windows over 512 columns come here
+  p.k =mode == 0 ? c->kmer_k : 0;
   for (int t = 0; t < 2; t++) p.kt[t] = KmerTable{c->d_kb[t].p, c->d_kk[t].p, c->d_kp[t].p, c->kmer_shift[t]};
   p.mask = c->d_smask.p; p.mask_words = mask_words; p.ckpt = c->d_ckpt.p; p.chunk_ids = c->d_chunk_ids.p;
   p.max_chunks = n_chunks; p.Lmax = Lmax; p.trace = c->d_strace.p;

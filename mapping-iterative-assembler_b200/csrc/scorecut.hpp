@@ -9,8 +9,10 @@
 // unless a / ulp is an exact tie.  A block of addends therefore moves S by ulp * sum(rint(a_i / ulp)) -- an integer
 // sum that any number of threads can take in any order -- provided no partial sum leaves the binade, which
 // N0 +- sum(|rint(a_i / ulp)|) bounds.  Blocks that fail the test (a binade crossing, a tie, the first few reads)
-// are added one read at a time exactly as the reference does.  tests/test_host_logic.py checks the result
-// against the plain chain and against the reference's own code.
+// are added one read at a time exactly as the reference does.  No test checks chained_sum() on its own:
+// tests/test_oracle_vs_ref.py (test_score_cut_matches_reference_regression) compares the whole cut, block path
+// included above 2,048 reads, with the oracle's plain chain on batches of up to 4,000 reads, and the session tests
+// compare the resulting dropped flags with the reference's.
 #pragma once
 #include <stdint.h>
 

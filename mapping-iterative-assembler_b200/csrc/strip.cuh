@@ -57,6 +57,7 @@ struct StripParams {
   int32_t len1;                       // columns (wrap_len if circular else seq_len)
   int32_t seq_len;
   const int32_t* prof;
+  int32_t sg5;                        // start-new level of a row (mia.c:877-880): 1 everywhere but miagpu_align_windows(..., sg5 = 0)
   int32_t k;                          // k-mer length, <= 0: no filter
   KmerTable kt[2];
   // per-warp scratch
@@ -114,7 +115,7 @@ __device__ __forceinline__ PV pv_better(PV a, PV b) { return (b.v > a.v) ? b : a
 // per-row {S1, S2, PV, PI}, ring_out = mine); the global checkpoints are still written, for the traceback.
 template <bool TRACE, bool PIPE = false, bool HP = false>
 __device__ void strip_chunk(const int L, const int len1, const int c0, const uint8_t* __restrict__ ref, const uint32_t* __restrict__ mask,
-                            const uint16_t* rowoff, const uint32_t prof_base, const int4* ck_in, const bool adjacent, const bool have_in,
+                            const uint16_t* rowoff, const uint32_t prof_base, const int sg5, const int4* ck_in, const bool adjacent, const bool have_in,
                             int4* ck_out, int32_t* trace, int& best, int& best_col, volatile int* flag_prev = nullptr,
                             volatile int* flag_mine = nullptr, volatile int* ring_in = nullptr, volatile int* ring_out = nullptr,
                             const HpChunk* hp = nullptr) {
@@ -177,7 +178,7 @@ __device__ void strip_chunk(const int L, const int len1, const int c0, const uin
   }
   for (int r = 1; r < L; r++) {
     const uint32_t pa = prof_base + rowoff[r];
-    const int N = -(GOP + GEP * (r + 1));                                // sg5 = 1 on every path that reaches here
+    const int N = sg5 ? -(GOP + GEP * (r + 1)) : 0;                      // mia.c:877-880
     // left neighbours of this lane's first column in row r-1
     int l1 = __shfl_up_sync(0xffffffffu, Sp[SK - 1], 1);
     int l2 = __shfl_up_sync(0xffffffffu, Sp[SK - 2], 1);
@@ -412,10 +413,10 @@ __device__ void strip_finish(const StripParams& p, const int rd, const int L, co
       __syncwarp();
       if (HP) {
         const HpChunk h = hp_chunk(p, *hprow, s, ws, len1, ids, q, ckh0 + (int64_t)s * (p.max_chunks + 1) * p.Lmax, false);
-        strip_chunk<true, false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, ck + (int64_t)q * p.Lmax,
+        strip_chunk<true, false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, p.sg5, ck + (int64_t)q * p.Lmax,
                                        q > 0 && ids[q - 1] == ch - 1, q > 0, nullptr, trace, dummy_b, dummy_c, nullptr, nullptr, nullptr, nullptr, &h);
       } else {
-        strip_chunk<true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, ck + (int64_t)q * p.Lmax,
+        strip_chunk<true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, p.sg5, ck + (int64_t)q * p.Lmax,
                           q > 0 && ids[q - 1] == ch - 1, q > 0, nullptr, trace, dummy_b, dummy_c);
       }
       __syncwarp();
@@ -574,10 +575,10 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) strip_kernel(StripParams
         const int ch = ids[q];
         if (HP) {
           const HpChunk h = hp_chunk(p, hprow, s, ws, len1, ids, q, ckh0 + (int64_t)s * (p.max_chunks + 1) * p.Lmax, true);
-          strip_chunk<false, false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, ck + (int64_t)q * p.Lmax, prev == ch - 1,
+          strip_chunk<false, false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, p.sg5, ck + (int64_t)q * p.Lmax, prev == ch - 1,
                                           q > 0, ck + (int64_t)(q + 1) * p.Lmax, nullptr, best[s], bcol[s], nullptr, nullptr, nullptr, nullptr, &h);
         } else {
-          strip_chunk<false>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, ck + (int64_t)q * p.Lmax, prev == ch - 1, q > 0,
+          strip_chunk<false>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, p.sg5, ck + (int64_t)q * p.Lmax, prev == ch - 1, q > 0,
                              ck + (int64_t)(q + 1) * p.Lmax, nullptr, best[s], bcol[s]);
         }
         prev = ch;
@@ -682,7 +683,7 @@ __global__ void __launch_bounds__(TEAM_WARPS * 32) strip_team_kernel(StripParams
       int wb = INT_MIN, wc = 0x7fffffff;
       for (int q = warp; q < n; q += TEAM_WARPS) {
         const int ch = ids[q];
-        strip_chunk<false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, ck + (int64_t)q * p.Lmax,
+        strip_chunk<false, true>(L, len1, ch * CW, p.ref_codes[s] + ws, mask, rowoff, prof_base, p.sg5, ck + (int64_t)q * p.Lmax,
                                  q > 0 && ids[q - 1] == ch - 1, q > 0, ck + (int64_t)(q + 1) * p.Lmax, nullptr, wb, wc,
                                  q > 0 ? s_flag + (q - 1) : nullptr, s_flag + q,
                                  s_ring + (size_t)((((q - 1) / TEAM_WARPS) & 1) * TEAM_WARPS + (q + TEAM_WARPS - 1) % TEAM_WARPS) * p.Lmax * 4,
