@@ -59,14 +59,7 @@ struct DevBuf {
 
 constexpr int NBUCKET = 10;                                  // 9 register-tiled widths + "big"
 static const int BUCKET_K[NBUCKET] = {2, 4, 5, 6, 7, 8, 10, 12, 16, 0};
-static const int P16_COLS[P16_NKB] = {128, 144, 160, 176, 192, 208, 224, 256, 64, 80, 96, 112};   // columns of the pair kernels' width classes
-// Lanes per pair in reiterate_assembly's windows with MIAGPU_PAIR_G=8: 8 lanes x 16..22 columns for the classes up to 176
-// columns (four pairs per warp, rows updated in place; the per-row scan and table build are shared by twice the cells:
-// 18 % fewer instructions per cell), 16 lanes beyond.  Measured on B200 it LOSES -- 1.47 vs 1.15 ms for the 160-column
-// class: 128 registers with spills and 16 warps per SM -- so the default is 16 lanes everywhere; the variant stays
-// selectable and tested (tests/test_gpu_pair16.py) as the starting point for a version with the table in registers.
-static const int P16_G_REALIGN[P16_NKB] = {8, 8, 8, 8, 16, 16, 16, 16, 16, 16, 16, 16};
-struct PairNp { int v[P16_NKB]; };                           // pairs per work item (= per warp) of every class
+constexpr int P16_COLS[P16_NKB] = {128, 144, 160, 176, 192, 208, 224, 256, 64, 80, 96, 112};   // columns of the pair kernels' width classes
 
 constexpr int MAX_CHUNKS = 16;
 constexpr int MAX_DEVICES = 64;
@@ -120,7 +113,7 @@ struct miagpu_ctx {
   DevBuf<int32_t> d_ckh;                       // one more checkpoint value per row and processed chunk (strip.cuh)
   cudaStream_t s_aux[4] = {};                  // [0] = stream; [1..3] side streams of the concurrent DP launches
   cudaEvent_t aev[8] = {};                     // fork / join events of those
-  cudaStream_t launch_stream = nullptr;        // where launch_bucket / launch_pair16 / launch_strip put their kernel
+  cudaStream_t launch_stream = nullptr;        // where launch_realign / launch_pair16 / launch_strip put their kernel
   int launch_slot = 0;
   // 16-bit SIMD pair kernel (pair16.cuh)
   DevBuf<int16_t> d_prof16;
@@ -132,7 +125,6 @@ struct miagpu_ctx {
   int32_t pair_reads[P16_NKB] = {}, pair_pairs[P16_NKB] = {};
   int64_t pair_cells[P16_NKB] = {};
   int32_t n_fallback = 0;
-  int pair_g = 16;
   // chunked pipeline of miagpu_iterate_host: upload / download streams, per-chunk events, pinned meta copies
   cudaStream_t s_up = nullptr, s_down = nullptr;
   cudaEvent_t cev[4 * 16] = {};                 // [MAX_CHUNKS][4]: classified, realigned, scores on host, spare
@@ -631,12 +623,12 @@ __global__ void classify_kernel(int64_t n, const int64_t* off, const int32_t* as
   if (direct) lists[(int64_t)b * n + s_base[b] + slot] = (int32_t)i;
 }
 
-// Pairs per (class, length) key: ceil(count / 2), rounded up to whole work items of np pairs (a warp's reads all
+// Pairs per (class, length) key: ceil(count / 2), rounded up to whole work items of P16_NP pairs (a warp's reads all
 // have one length), laid out class after class.  META_PSTART is in pairs, META_NPAIRS in work items.
 // One block: a thread takes LAYOUT_PER consecutive keys, the block scans the per-thread totals.
 constexpr int LAYOUT_THREADS = 256;
 constexpr int LAYOUT_PER = (P16_KEYS + LAYOUT_THREADS - 1) / LAYOUT_THREADS;
-__global__ void __launch_bounds__(LAYOUT_THREADS) pair_layout_kernel(int32_t* meta, PairNp npk) {
+__global__ void __launch_bounds__(LAYOUT_THREADS) pair_layout_kernel(int32_t* meta) {
   __shared__ int s_tot[LAYOUT_THREADS];
   __shared__ int s_start[P16_KEYS + 1];
   const int t = threadIdx.x;
@@ -645,8 +637,7 @@ __global__ void __launch_bounds__(LAYOUT_THREADS) pair_layout_kernel(int32_t* me
   for (int q = 0; q < LAYOUT_PER; q++) {
     const int k = t * LAYOUT_PER + q;
     const int pairs = k < P16_KEYS ? (meta[META_HIST + k] + 1) >> 1 : 0;
-    const int np = npk.v[min(k / (P16_MAXL + 1), P16_NKB - 1)];
-    items[q] = (pairs + np - 1) / np * np;
+    items[q] = (pairs + P16_NP - 1) / P16_NP * P16_NP;
     sum += items[q];
   }
   s_tot[t] = sum;
@@ -666,7 +657,7 @@ __global__ void __launch_bounds__(LAYOUT_THREADS) pair_layout_kernel(int32_t* me
   }
   if (t == LAYOUT_THREADS - 1) s_start[P16_KEYS] = s_tot[t];
   __syncthreads();
-  if (t < P16_NKB) meta[META_NPAIRS + t] = (s_start[(t + 1) * (P16_MAXL + 1)] - s_start[t * (P16_MAXL + 1)]) / npk.v[t];
+  if (t < P16_NKB) meta[META_NPAIRS + t] = (s_start[(t + 1) * (P16_MAXL + 1)] - s_start[t * (P16_MAXL + 1)]) / P16_NP;
 }
 
 // Eligible reads take the next free slot of their key: slot s is member s&1 of pair pstart + s/2.
@@ -794,59 +785,35 @@ static int launch_strip(miagpu_ctx* c, int mode, const int32_t* list, int n_list
   return 1;
 }
 
-template <int K>
-static int launch_bucket(miagpu_ctx* c, RealignParams p, int maxL) {
-  using TL = TraceLayout<K>;
-  bool ref_in_smem = c->ref_bytes <= 160 * 1024;
-  size_t smem = PROF_INTS * 4 + WARPS_PER_BLOCK * MAX_READ * 2 + (ref_in_smem ? c->ref_bytes : 0);
-  // per instantiation AND per device (function attributes belong to a device; several contexts of one process may drive several GPUs):
-  // the attribute / occupancy calls cost more than the launch
+// Blocks of KERNEL one SM holds with `smem` bytes of dynamic shared memory; 0 with the error set when the kernel does not fit or a
+// CUDA call fails.  Cached per instantiation AND per device (function attributes belong to a device; several contexts of one process
+// may drive several GPUs): the attribute / occupancy calls cost more than the launch.
+template <auto KERNEL>
+static int blocks_per_sm(miagpu_ctx* c, size_t smem, const char* name, int K) {
   static size_t cached_smem_d[MAX_DEVICES];
   static int cached_per_sm_d[MAX_DEVICES];
   size_t& cached_smem = cached_smem_d[c->device % MAX_DEVICES];
   int& cached_per_sm = cached_per_sm_d[c->device % MAX_DEVICES];
   if (cached_smem != smem + 1) {
-    MIAGPU_CUDA(cudaFuncSetAttribute(realign_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MIAGPU_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm, realign_kernel<K>, WARPS_PER_BLOCK * 32, smem));
+    MIAGPU_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MIAGPU_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm, KERNEL, WARPS_PER_BLOCK * 32, smem));
     cached_smem = smem + 1;
   }
-  int per_sm = cached_per_sm;
-  if (per_sm < 1) { set_error("realign_kernel<%d> does not fit on an SM (smem %zu)", K, smem); return 0; }
-  int cap = 8;                                             // 32 warps/SM (measured best on B200); bounds the trace scratch
-  if (const char* e = getenv("MIAGPU_BLOCKS_PER_SM")) cap = std::max(1, atoi(e));
-  per_sm = std::min(per_sm, cap);
-  int blocks = c->num_sms * per_sm;
-  blocks = std::min(blocks, (p.n_list + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
-  if (blocks < 1) return 1;
-  int64_t words = (int64_t)std::max(maxL - 1, 1) * TL::ROW_WORDS;
-  DevBuf<uint32_t>& scratch = c->d_scratch[c->launch_slot];
-  if (!scratch.reserve((size_t)words * blocks * WARPS_PER_BLOCK)) return 0;
-  p.scratch = scratch.p;
-  p.scratch_words_per_warp = words;
-  p.ref_in_smem = ref_in_smem;
-  realign_kernel<K><<<blocks, WARPS_PER_BLOCK * 32, smem, c->launch_stream>>>(p);
-  MIAGPU_CUDA(cudaGetLastError());
-  c->launches++;
-  return 1;
+  if (cached_per_sm < 1) set_error("%s<%d> does not fit on an SM (smem %zu)", name, K, smem);
+  return std::max(cached_per_sm, 0);
 }
 
-// pass 1: the winning jobs whose path is not one plain diagonal, stretch by stretch with a trace (realign.cuh, JOB)
-template <int K>
-static int launch_p1_trace(miagpu_ctx* c, RealignParams p, int maxL) {
+// realign_kernel over a work list: a width bucket of reiterate_assembly's windows (JOB = false), or pass 1's winning jobs whose
+// path is not one plain diagonal, stretch by stretch with a trace (JOB = true)
+template <int K, bool JOB = false>
+static int launch_realign(miagpu_ctx* c, RealignParams p, int maxL) {
   using TL = TraceLayout<K>;
   const bool ref_in_smem = p.ref_bytes <= 160 * 1024;
   const size_t smem = PROF_INTS * 4 + WARPS_PER_BLOCK * MAX_READ * 2 + (ref_in_smem ? p.ref_bytes : 0);
-  static size_t cached_smem_d[MAX_DEVICES];
-  static int cached_per_sm_d[MAX_DEVICES];
-  size_t& cached_smem = cached_smem_d[c->device % MAX_DEVICES];
-  int& cached_per_sm = cached_per_sm_d[c->device % MAX_DEVICES];
-  if (cached_smem != smem + 1) {
-    MIAGPU_CUDA(cudaFuncSetAttribute((realign_kernel<K, false, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MIAGPU_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm, (realign_kernel<K, false, true>), WARPS_PER_BLOCK * 32, smem));
-    cached_smem = smem + 1;
-  }
-  if (cached_per_sm < 1) { set_error("realign_kernel<%d, JOB> does not fit on an SM (smem %zu)", K, smem); return 0; }
-  const int blocks = std::min(c->num_sms * std::min(cached_per_sm, 8), (p.n_list + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
+  const int per_sm = blocks_per_sm<realign_kernel<K, false, JOB>>(c, smem, JOB ? "realign_kernel (pass-1 jobs)" : "realign_kernel", K);
+  if (per_sm < 1) return 0;
+  // at most 8 blocks = 32 warps per SM (measured best on B200); bounds the trace scratch
+  const int blocks = std::min(c->num_sms * std::min(per_sm, 8), (p.n_list + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
   if (blocks < 1) return 1;
   const int64_t words = (int64_t)std::max(maxL - 1, 1) * TL::ROW_WORDS;
   DevBuf<uint32_t>& scratch = c->d_scratch[c->launch_slot];
@@ -854,40 +821,49 @@ static int launch_p1_trace(miagpu_ctx* c, RealignParams p, int maxL) {
   p.scratch = scratch.p;
   p.scratch_words_per_warp = words;
   p.ref_in_smem = ref_in_smem;
-  realign_kernel<K, false, true><<<blocks, WARPS_PER_BLOCK * 32, smem, c->launch_stream>>>(p);
+  realign_kernel<K, false, JOB><<<blocks, WARPS_PER_BLOCK * 32, smem, c->launch_stream>>>(p);
   MIAGPU_CUDA(cudaGetLastError());
   c->launches++;
   return 1;
 }
 
-template <int K, int G, bool JOB = false, bool RB = false>
-static int launch_pair16(miagpu_ctx* c, Pair16Params p, int n_pairs, int maxL) {
-  bool ref_in_smem = p.ref_bytes <= 160 * 1024;
-  size_t smem = p16_smem_fixed<G>() + (ref_in_smem ? p.ref_bytes : 0);
-  static size_t cached_smem_d[MAX_DEVICES];
-  static int cached_per_sm_d[MAX_DEVICES];
-  size_t& cached_smem = cached_smem_d[c->device % MAX_DEVICES];
-  int& cached_per_sm = cached_per_sm_d[c->device % MAX_DEVICES];
-  if (cached_smem != smem + 1) {
-    MIAGPU_CUDA(cudaFuncSetAttribute((pair16_kernel<K, G, JOB, RB>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MIAGPU_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cached_per_sm, (pair16_kernel<K, G, JOB, RB>), WARPS_PER_BLOCK * 32, smem));
-    cached_smem = smem + 1;
-  }
+template <int K, bool JOB, bool RB>
+static int launch_pair16(miagpu_ctx* c, Pair16Params p, int n_items) {
+  const bool ref_in_smem = p.ref_bytes <= 160 * 1024;
+  const size_t smem = P16_SMEM_FIXED + (ref_in_smem ? p.ref_bytes : 0);
+  const int per_sm = blocks_per_sm<pair16_kernel<K, JOB, RB>>(c, smem, "pair16_kernel", K);
+  if (per_sm < 1) return 0;
   if (RB) { const RbFrame f = p16_rb_frame(K, c->pssm_max); p.rb_off = f.off; p.rb_d = f.d; p.rb_thresh = f.thresh; }
-  int per_sm = cached_per_sm;
-  if (per_sm < 1) { set_error("pair16_kernel<%d,%d> does not fit on an SM (smem %zu)", K, G, smem); return 0; }
-  int cap = 8;
-  if (const char* e = getenv("MIAGPU_PAIR_BLOCKS_PER_SM")) cap = std::max(1, atoi(e));
-  per_sm = std::min(per_sm, cap);
-  int blocks = std::min(c->num_sms * per_sm, (n_pairs + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
+  const int blocks = std::min(c->num_sms * std::min(per_sm, 8), (n_items + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK);
   if (blocks < 1) return 1;
-  (void)maxL;
   p.ref_in_smem = ref_in_smem;
   p.gep2 = K2(2 * GEP);
-  pair16_kernel<K, G, JOB, RB><<<blocks, WARPS_PER_BLOCK * 32, smem, c->launch_stream>>>(p);
+  pair16_kernel<K, JOB, RB><<<blocks, WARPS_PER_BLOCK * 32, smem, c->launch_stream>>>(p);
   MIAGPU_CUDA(cudaGetLastError());
   c->launches++;
   return 1;
+}
+
+// is pair class kb built in the RB frame (pair16.cuh 5.)?  The wide classes only (K = 8 .. 16); for pass-1 jobs K = 10 .. 16 (a
+// stretch is about L + 20 columns)
+constexpr bool pair_rb_built(int kb, bool job) { return kb < P16_NKB_WIDE && !(job && kb < 2); }
+
+// The pair kernel of class kb in the low or the RB frame.  Realign windows use the wide classes only; pass-1 jobs also the narrow
+// ones, in the low frame.  A (class, frame) without a kernel is an error.
+template <bool JOB, int KB = 0>
+static int launch_pair_class(miagpu_ctx* c, const Pair16Params& p, int kb, bool rb, int n_items) {
+  if constexpr (KB < P16_NKB) {
+    if (kb != KB) return launch_pair_class<JOB, KB + 1>(c, p, kb, rb, n_items);
+    constexpr int K = P16_COLS[KB] / P16_G;
+    if constexpr (JOB || KB < P16_NKB_WIDE) {
+      if (!rb) return launch_pair16<K, JOB, false>(c, p, n_items);
+    }
+    if constexpr (pair_rb_built(KB, JOB)) {
+      if (rb) return launch_pair16<K, JOB, true>(c, p, n_items);
+    }
+  }
+  set_error("pair class %d has no %s kernel in the %s frame", kb, JOB ? "pass-1 job" : "realign window", rb ? "RB" : "low");
+  return 0;
 }
 
 // One realign job = reads [lo, lo + n) of the resident batch with their own meta block, work lists and pair
@@ -921,29 +897,19 @@ static void pick_stream(miagpu_ctx* c, bool concurrent, int& rr) {
   c->launch_stream = c->s_aux[c->launch_slot];
 }
 
-static int realign_g(int kb) {
-  const char* e = getenv("MIAGPU_PAIR_G");
-  return (e && atoi(e) == 8) ? P16_G_REALIGN[kb] : 16;
-}
-static PairNp realign_np() {
-  PairNp r;
-  for (int kb = 0; kb < P16_NKB; kb++) r.v[kb] = 32 / realign_g(kb);
-  return r;
-}
 // longest read every pair class takes in the low frame (pair16.cuh 2.)
 static PairLmax pair_lmax_low(miagpu_ctx* c) {
   int lmax16 = c->lmax16;
   if (const char* e = getenv("MIAGPU_PAIR16")) if (atoi(e) == 0) lmax16 = 0;
-  c->pair_g = 16;                                    // lanes per pair of the pass-1 job kernels
   PairLmax lm{};
-  for (int kb = 0; kb < P16_NKB; kb++) lm.v[kb] = lmax16 > 0 ? std::min(p16_lmax(P16_COLS[kb] / realign_g(kb), c->pssm_max), P16_MAXL) : 0;
+  for (int kb = 0; kb < P16_NKB; kb++) lm.v[kb] = lmax16 > 0 ? std::min(p16_lmax(P16_COLS[kb] / P16_G, c->pssm_max), P16_MAXL) : 0;
   return lm;
 }
-// does the class have an RB instantiation (pair16.cuh 5.) with room for real reads under the current matrices?
+// does the class have an RB instantiation with room for real reads under the current matrices?
 static bool pair_rb_class(miagpu_ctx* c, int kb, bool job) {
   if (const char* e = getenv("MIAGPU_PAIR_RB")) if (atoi(e) == 0) return false;
-  if (realign_g(kb) != 16 || kb >= P16_NKB_WIDE || (job && kb < 2)) return false;      // JOB: K = 10 .. 16 only (a stretch is about L + 20 columns)
-  return p16_rb_frame(P16_COLS[kb] / 16, c->pssm_max).room >= 16384;
+  if (!pair_rb_built(kb, job)) return false;
+  return p16_rb_frame(P16_COLS[kb] / P16_G, c->pssm_max).room >= 16384;
 }
 // longest read every pair class takes at all: the RB frame holds any read of the class's width
 static PairLmax pair_lmax(miagpu_ctx* c, bool job = false) {
@@ -973,7 +939,7 @@ static int realign_classify(miagpu_ctx* c, const RealignJob& j, cudaStream_t st)
   MIAGPU_CUDA(cudaGetLastError());
   c->launches++;
   if (lm.v[0] > 0) {
-    pair_layout_kernel<<<1, LAYOUT_THREADS, 0, st>>>(j.d_meta, realign_np());
+    pair_layout_kernel<<<1, LAYOUT_THREADS, 0, st>>>(j.d_meta);
     MIAGPU_CUDA(cudaGetLastError());
     c->launches++;
   }
@@ -986,7 +952,6 @@ static int realign_launch(miagpu_ctx* c, const RealignJob& j) {
   const int64_t n = j.n, lo = j.lo;
   if (n == 0) return 1;
   const int32_t* meta = j.h_meta;
-  const PairNp npk = realign_np();
   const PairLmax lm_low = pair_lmax_low(c);
   const bool concurrent = !j.timed && !getenv("MIAGPU_SERIAL_LAUNCH") && !c->hp;     // the chunked kernel's launches share their scratch
   int rr = 0;
@@ -995,11 +960,11 @@ static int realign_launch(miagpu_ctx* c, const RealignJob& j) {
   memcpy(pcells, meta + META_PCELLS, sizeof(pcells));
   for (int b = 0; b < NBUCKET; b++) { c->bucket_cells[b] += cells[b]; c->dp_cells += cells[b]; }
   int pair_items[P16_NKB];
-  int total_pairs = 0;                               // pair slots of all classes (a work item holds npk.v[class] pairs)
+  int total_pairs = 0;                               // pair slots of all classes (a work item holds P16_NP pairs)
   for (int kb = 0; kb < P16_NKB; kb++) {
     pair_items[kb] = meta[META_NPAIRS + kb];
     c->pair_pairs[kb] += pair_items[kb]; c->pair_reads[kb] += meta[META_PREADS + kb]; c->pair_cells[kb] += pcells[kb];
-    total_pairs += pair_items[kb] * npk.v[kb];
+    total_pairs += pair_items[kb] * P16_NP;
   }
 
   // ---- 16-bit pair kernels first: the reads they cannot finish join the 32-bit lists
@@ -1009,7 +974,7 @@ static int realign_launch(miagpu_ctx* c, const RealignJob& j) {
     MIAGPU_CUDA(cudaGetLastError());
     c->launches++;
     int base_of[P16_NKB], base = 0, order[P16_NKB];
-    for (int kb = 0; kb < P16_NKB; kb++) { base_of[kb] = base; base += pair_items[kb] * npk.v[kb]; order[kb] = kb; }   // in pair slots
+    for (int kb = 0; kb < P16_NKB; kb++) { base_of[kb] = base; base += pair_items[kb] * P16_NP; order[kb] = kb; }   // in pair slots
     if (concurrent) {                                 // biggest class first: the small ones fill its tail
       std::sort(order, order + P16_NKB, [&](int a, int b) { return pcells[a] > pcells[b]; });
       if (!fork_streams(c, 0)) return 0;
@@ -1029,33 +994,8 @@ static int realign_launch(miagpu_ctx* c, const RealignJob& j) {
       p.score = c->d_score.p + lo; p.as_out = c->d_as_out.p + lo; p.ae_out = c->d_ae_out.p + lo; p.abr = c->d_abr.p + lo;
       p.n_runs = c->d_nruns.p + lo; p.runs = c->d_runs.p + lo * MAX_RUNS; p.status = c->d_status.p + lo;
       p.lists = j.d_lists; p.list_counts = j.d_meta + META_COUNT; p.n_reads = n; p.n_fallback = j.d_meta + META_NFALL;
-      const int maxL = P16_MAXL;
-      int ok = 1;
       const bool rb = meta[META_PMAXL + kb] > lm_low.v[kb];         // a read of the class is beyond the low frame: the whole class takes the RB frame
-      switch (realign_g(kb) == 8 ? 100 + kb : rb ? 200 + kb : kb) {
-        case 200: ok = launch_pair16<8, 16, false, true>(c, p, ni, maxL); break;
-        case 201: ok = launch_pair16<9, 16, false, true>(c, p, ni, maxL); break;
-        case 202: ok = launch_pair16<10, 16, false, true>(c, p, ni, maxL); break;
-        case 203: ok = launch_pair16<11, 16, false, true>(c, p, ni, maxL); break;
-        case 204: ok = launch_pair16<12, 16, false, true>(c, p, ni, maxL); break;
-        case 205: ok = launch_pair16<13, 16, false, true>(c, p, ni, maxL); break;
-        case 206: ok = launch_pair16<14, 16, false, true>(c, p, ni, maxL); break;
-        case 207: ok = launch_pair16<16, 16, false, true>(c, p, ni, maxL); break;
-        case 100: ok = launch_pair16<16, 8>(c, p, ni, maxL); break;
-        case 101: ok = launch_pair16<18, 8>(c, p, ni, maxL); break;
-        case 102: ok = launch_pair16<20, 8>(c, p, ni, maxL); break;
-        case 103: ok = launch_pair16<22, 8>(c, p, ni, maxL); break;
-        case 0: ok = launch_pair16<8, 16>(c, p, ni, maxL); break;
-        case 1: ok = launch_pair16<9, 16>(c, p, ni, maxL); break;
-        case 2: ok = launch_pair16<10, 16>(c, p, ni, maxL); break;
-        case 3: ok = launch_pair16<11, 16>(c, p, ni, maxL); break;
-        case 4: ok = launch_pair16<12, 16>(c, p, ni, maxL); break;
-        case 5: ok = launch_pair16<13, 16>(c, p, ni, maxL); break;
-        case 6: ok = launch_pair16<14, 16>(c, p, ni, maxL); break;
-        case 7: ok = launch_pair16<16, 16>(c, p, ni, maxL); break;
-        default: set_error("pair class %d holds no realign window", kb); ok = 0; break;
-      }
-      if (!ok) return 0;
+      if (!launch_pair_class<false>(c, p, kb, rb, ni)) return 0;
       if (j.timed) MIAGPU_CUDA(cudaEventRecord(c->pev[2 * kb + 1], c->stream));
     }
     if (concurrent && !join_streams(c, 0)) return 0;
@@ -1100,15 +1040,15 @@ static int realign_launch(miagpu_ctx* c, const RealignJob& j) {
       continue;
     }
     switch (BUCKET_K[b]) {
-      case 2: ok = launch_bucket<2>(c, p, maxL); break;
-      case 4: ok = launch_bucket<4>(c, p, maxL); break;
-      case 5: ok = launch_bucket<5>(c, p, maxL); break;
-      case 6: ok = launch_bucket<6>(c, p, maxL); break;
-      case 7: ok = launch_bucket<7>(c, p, maxL); break;
-      case 8: ok = launch_bucket<8>(c, p, maxL); break;
-      case 10: ok = launch_bucket<10>(c, p, maxL); break;
-      case 12: ok = launch_bucket<12>(c, p, maxL); break;
-      case 16: ok = launch_bucket<16>(c, p, maxL); break;
+      case 2: ok = launch_realign<2>(c, p, maxL); break;
+      case 4: ok = launch_realign<4>(c, p, maxL); break;
+      case 5: ok = launch_realign<5>(c, p, maxL); break;
+      case 6: ok = launch_realign<6>(c, p, maxL); break;
+      case 7: ok = launch_realign<7>(c, p, maxL); break;
+      case 8: ok = launch_realign<8>(c, p, maxL); break;
+      case 10: ok = launch_realign<10>(c, p, maxL); break;
+      case 12: ok = launch_realign<12>(c, p, maxL); break;
+      case 16: ok = launch_realign<16>(c, p, maxL); break;
       default:
         ok = launch_strip(c, 2, p.list, meta[META_COUNT + b], j.d_meta + META_WORK + b, lo);   // too wide for either kernel (its window, or the whole reference, as the matrix): never pair-eligible
     }
@@ -1253,7 +1193,7 @@ extern "C" int miagpu_last_buckets(miagpu_ctx* c, int32_t* k, int32_t* reads, in
 extern "C" int miagpu_last_pair_buckets(miagpu_ctx* c, int32_t* k, int32_t* reads, int32_t* pairs, int64_t* cells, float* ms, int32_t* fallback_reads, int32_t* max_len16) {
   if (!c) { set_error("miagpu_last_pair_buckets: NULL ctx"); return 0; }
   for (int kb = 0; kb < P16_NKB_WIDE; kb++) {            // MIAGPU_NPAIRCLASS slots: the classes realign windows use
-    if (k) k[kb] = P16_COLS[kb] / realign_g(kb);
+    if (k) k[kb] = P16_COLS[kb] / P16_G;
     if (reads) reads[kb] = c->pair_reads[kb];
     if (pairs) pairs[kb] = c->pair_pairs[kb];
     if (cells) cells[kb] = c->pair_cells[kb];
@@ -3490,7 +3430,6 @@ static int launch_sweep(miagpu_ctx* c, const int32_t* jobs, int64_t m, int lmax_
 static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
   const PairLmax lm_low = pair_lmax_low(c);
   const int64_t n = c->n, nj = 10 * n + 4096;          // job capacity; reads whose jobs do not fit go to the general kernel
-  const int np = 32 / c->pair_g;
   if (n > 0x7fffffffLL / 8) { set_error("miagpu_pass1: at most %d reads per batch", 0x7fffffff / 8); return 0; }
   if (!c->d_jread.reserve(nj + 1) || !c->d_jfirst.reserve(n + 1) || !c->d_jcount.reserve(n + 1)) return 0;
   if (!c->d_jkind.reserve(nj + 1) || !c->d_jstatus.reserve(nj + 1) || !c->d_route.reserve(n + 1) || !c->d_jws.reserve(nj + 1) ||
@@ -3513,8 +3452,7 @@ static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
   const unsigned seed_blocks = (unsigned)std::min<int64_t>((int64_t)c->num_sms * 8, (n + 7) / 8);
   p1_seed_kernel<<<seed_blocks, 256, 0, st>>>(sp);
   MIAGPU_CUDA(cudaGetLastError());
-  PairNp npj; for (int kb = 0; kb < P16_NKB; kb++) npj.v[kb] = np;
-  pair_layout_kernel<<<1, LAYOUT_THREADS, 0, st>>>(meta, npj);
+  pair_layout_kernel<<<1, LAYOUT_THREADS, 0, st>>>(meta);
   MIAGPU_CUDA(cudaGetLastError());
   MIAGPU_CUDA(cudaEventRecord(c->p1ev[0], st));
   MIAGPU_CUDA(cudaMemcpyAsync(c->h_meta, meta, sizeof(int32_t) * META_HOST, cudaMemcpyDeviceToHost, st));
@@ -3541,7 +3479,7 @@ static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
     MIAGPU_CUDA(cudaEventRecord(c->aev[1], c->s_aux[1]));
   }
   if (total_pairs) {
-    MIAGPU_CUDA(cudaMemsetAsync(c->d_jpairs.p, 0xff, (size_t)2 * np * total_pairs * sizeof(int32_t), st));
+    MIAGPU_CUDA(cudaMemsetAsync(c->d_jpairs.p, 0xff, (size_t)2 * P16_NP * total_pairs * sizeof(int32_t), st));
     const int64_t njobs = std::min<int64_t>(nj, (uint32_t)c->h_meta[P1_NJOBS]);
     pair_scatter_kernel<<<(unsigned)((njobs + 255) / 256), 256, 0, st>>>(njobs, c->d_off.p, c->d_jkind.p, meta, c->d_jpairs.p, c->d_jread.p);
     MIAGPU_CUDA(cudaGetLastError());
@@ -3561,34 +3499,13 @@ static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
       c->launch_stream = lanes3[rr++ % 3];
       Pair16Params p{};
       p.bases = c->d_bases.p; p.off = c->d_off.p; p.rc = nullptr; p.win_start = c->d_jws.p; p.win_len = c->d_jwl.p;
-      p.pairs = c->d_jpairs.p + 2 * (int64_t)np * base; p.n_items = meta + META_NPAIRS + kb; p.counter = meta + META_PWORK + kb;
+      p.pairs = c->d_jpairs.p + 2 * (int64_t)P16_NP * base; p.n_items = meta + META_NPAIRS + kb; p.counter = meta + META_PWORK + kb;
       p.ref_codes = c->d_ref2.p; p.ref_bytes = 2 * c->ref_bytes; p.strand_stride = c->ref_bytes; p.prof16 = c->d_prof16.p; p.job_read = c->d_jread.p;
       p.score = c->d_jscore.p; p.as_out = c->d_jabc.p; p.ae_out = c->d_jaec.p; p.abr = c->d_jabr.p; p.status = c->d_jstatus.p;
       p.n_reads = nj;
       p.sunk_list = c->d_p1sunk.p; p.sunk_count = meta + P1_NSUNK;
-      int ok = 1;
       const bool rb = c->h_meta[META_PMAXL + kb] > lm_low.v[kb];
-      switch (rb ? 200 + kb : kb) {
-        case 202: ok = launch_pair16<10, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 203: ok = launch_pair16<11, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 204: ok = launch_pair16<12, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 205: ok = launch_pair16<13, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 206: ok = launch_pair16<14, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 207: ok = launch_pair16<16, 16, true, true>(c, p, ni, P16_MAXL); break;
-        case 0: ok = launch_pair16<8, 16, true>(c, p, ni, P16_MAXL); break;
-        case 1: ok = launch_pair16<9, 16, true>(c, p, ni, P16_MAXL); break;
-        case 2: ok = launch_pair16<10, 16, true>(c, p, ni, P16_MAXL); break;
-        case 3: ok = launch_pair16<11, 16, true>(c, p, ni, P16_MAXL); break;
-        case 4: ok = launch_pair16<12, 16, true>(c, p, ni, P16_MAXL); break;
-        case 5: ok = launch_pair16<13, 16, true>(c, p, ni, P16_MAXL); break;
-        case 6: ok = launch_pair16<14, 16, true>(c, p, ni, P16_MAXL); break;
-        case 7: ok = launch_pair16<16, 16, true>(c, p, ni, P16_MAXL); break;
-        case 8: ok = launch_pair16<4, 16, true>(c, p, ni, P16_MAXL); break;
-        case 9: ok = launch_pair16<5, 16, true>(c, p, ni, P16_MAXL); break;
-        case 10: ok = launch_pair16<6, 16, true>(c, p, ni, P16_MAXL); break;
-        default: ok = launch_pair16<7, 16, true>(c, p, ni, P16_MAXL); break;
-      }
-      if (!ok) { c->launch_stream = st; return 0; }
+      if (!launch_pair_class<true>(c, p, kb, rb, ni)) { c->launch_stream = st; return 0; }
       base += ni;
     }
     c->launch_stream = st;
@@ -3614,7 +3531,7 @@ static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
       p.counter = meta + P1_SWORK + t;
       p.job_wl_lo = t == 0 ? 0 : t == 1 ? 64 : 128;
       p.job_wl_hi = t == 0 ? 64 : t == 1 ? 128 : 256;
-      const int ok = t == 0 ? launch_p1_trace<2>(c, p, maxL) : t == 1 ? launch_p1_trace<4>(c, p, maxL) : launch_p1_trace<8>(c, p, maxL);
+      const int ok = t == 0 ? launch_realign<2, true>(c, p, maxL) : t == 1 ? launch_realign<4, true>(c, p, maxL) : launch_realign<8, true>(c, p, maxL);
       if (!ok) { c->launch_slot = 0; return 0; }
     }
     c->launch_slot = 0;
@@ -3660,7 +3577,7 @@ static int pass1_fast(miagpu_ctx* c, const PairLmax& lm) {
       p.counter = meta + P1_TWORK + t;
       p.job_wl_lo = t == 0 ? 0 : t == 1 ? 64 : 128;
       p.job_wl_hi = t == 0 ? 64 : t == 1 ? 128 : 256;
-      ok = t == 0 ? launch_p1_trace<2>(c, p, maxL) : t == 1 ? launch_p1_trace<4>(c, p, maxL) : launch_p1_trace<8>(c, p, maxL);
+      ok = t == 0 ? launch_realign<2, true>(c, p, maxL) : t == 1 ? launch_realign<4, true>(c, p, maxL) : launch_realign<8, true>(c, p, maxL);
     }
     c->launch_stream = st; c->launch_slot = 0;
     if (!ok) return 0;

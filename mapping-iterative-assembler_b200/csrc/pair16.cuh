@@ -7,10 +7,10 @@
 // diagonal.  Everything else is handed, read by read, to the 32-bit kernel of realign.cuh through
 // its work list -- never approximated.
 //
-// 1. Two reads of equal length share a group of G lanes: every 32-bit register holds the same DP
+// 1. Two reads of equal length share a group of 16 lanes: every 32-bit register holds the same DP
 //    cell of read A (low half) and read B (high half), so one VIADDMNMX.U16x2 / VIMNMX3.U16x2 does
-//    two cells.  Lane l of the group owns columns [l*K, l*K+K) as in realign.cuh.  G = 16: a warp
-//    carries two such pairs (four reads of equal length).
+//    two cells.  Lane l of the group owns columns [l*K, l*K+K) as in realign.cuh.  A warp carries
+//    two such pairs (four reads of equal length).
 //
 // 2. Lane frame (checked lane for lane against the oracle by tests/model/pair16_model.c).  A cell of
 //    column c = l*K + j is held as  V(r,c) = S(r,c) + GEP*r + GEP*j - OFF  (stored biased, V + 32768,
@@ -65,6 +65,8 @@ constexpr int P16_NKB = 12;                         // width classes: 128 / 144 
                                                     // then the narrow classes of pass-1 jobs: 64 / 80 / 96 / 112 (K = 4 .. 7)
 constexpr int P16_NKB_WIDE = 8;                     // classes reiterate_assembly's windows use (a window is at least 100 columns + the read)
 constexpr int P16_TAB_WORDS = 64;                   // 25 64-bit entries, padded to 32
+constexpr int P16_G = 16;                           // lanes per pair (1. in the header)
+constexpr int P16_NP = 32 / P16_G;                  // pairs per warp = per work item
 
 // OFF of the lane frame: the lowest intermediate, (lowest cell = -OFF-GOP-GEP+min entry) converted to the next lane
 // (-GEP*K) minus GOP, must stay above -32768 for every matrix set_pssm accepts (|entry| <= PSSM_ABS_LIMIT).
@@ -118,7 +120,7 @@ struct Pair16Params {
   const int32_t* win_start;
   const int32_t* win_len;
   int32_t* win_len_narrow;       // realign windows only (null = off): a read handed to the 32-bit kernels keeps the columns up to its end cell
-  const int32_t* pairs;          // [n_items][32/G][2] read ids; -1 = empty slot (a work item's first slot is never empty)
+  const int32_t* pairs;          // [n_items][P16_NP][2] read ids; -1 = empty slot (a work item's first slot is never empty)
   const int32_t* n_items;        // device counter (layout kernel wrote it)
   int32_t* counter;
   const uint8_t* ref_codes;
@@ -209,11 +211,8 @@ __device__ __forceinline__ uint32_t cell_pair(uint32_t best, uint32_t ncmp, uint
   return w;
 }
 
-// dynamic shared memory: [prof16 (PROF16_N + 8) int16][rowoff WARPS*(32/G)*2*P16_MAXL u16][tab WARPS*(32/G)*2*32 u32][ref codes]
-template <int G>
-__host__ __device__ constexpr int p16_smem_fixed() {
-  return (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * (32 / G) * 2 * P16_MAXL * 2 + WARPS_PER_BLOCK * (32 / G) * 2 * P16_TAB_WORDS * 4;
-}
+// dynamic shared memory: [prof16 (PROF16_N + 8) int16][rowoff WARPS*P16_NP*2*P16_MAXL u16][tab WARPS*P16_NP*2*P16_TAB_WORDS u32][ref codes]
+constexpr int P16_SMEM_FIXED = (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * P16_NP * 2 * P16_MAXL * 2 + WARPS_PER_BLOCK * P16_NP * 2 * P16_TAB_WORDS * 4;
 
 // JOB = false: a work item names reads (reiterate_assembly's windows, matrix by strand).
 // JOB = true : pass 1 with the k-mer filter (sg_align, mia.c:1500-1610).  A work item names jobs (pass1.cuh;
@@ -223,35 +222,25 @@ __host__ __device__ constexpr int p16_smem_fixed() {
 //   (S = N, substitution score not added, mia.c:910-915) instead of applying the column-0 rule (mia.c:805-822).
 //   Everything to the left / right of the stretch is HIM and can neither be chosen nor become the best end cell.
 //   Outputs are per job, in strand coordinates: as_out = abc, ae_out = aec.
-#ifndef P16_INPLACE
-#define P16_INPLACE 0
-#endif
-#ifndef P16_SCAN4
-#define P16_SCAN4 0
-#endif
-#ifndef P16_SIX_BLOCKS_K
-#define P16_SIX_BLOCKS_K 7
-#endif
-template <int K, int G, bool JOB, bool RB = false>
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_SIX_BLOCKS_K ? 6 : K <= 12 ? 5 : 4)) pair16_kernel(Pair16Params p) {
-  static_assert(K >= 4 && ((G == 16 && K <= 16) || (G == 8 && K <= 24)), "columns per lane / lanes per pair");
-  constexpr int NP = 32 / G;                         // pairs per warp
-  constexpr int NE = (25 + G - 1) / G;               // table entries a lane builds per row
+template <int K, bool JOB, bool RB = false>
+__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= 7 ? 6 : K <= 12 ? 5 : 4)) pair16_kernel(Pair16Params p) {
+  static_assert(K >= 4 && K <= 16, "columns per lane");
+  constexpr int NE = (25 + P16_G - 1) / P16_G;       // table entries a lane builds per row
   extern __shared__ __align__(16) uint8_t smem[];
   __shared__ __align__(8) uint64_t ref_bar;
   int16_t* s_prof = reinterpret_cast<int16_t*>(smem);
   constexpr int PROF_BYTES = (PROF16_N + 8) * 2;
-  constexpr int ROWOFF_BYTES = WARPS_PER_BLOCK * NP * 2 * P16_MAXL * 2;
+  constexpr int ROWOFF_BYTES = WARPS_PER_BLOCK * P16_NP * 2 * P16_MAXL * 2;
   uint16_t* s_rowoff = reinterpret_cast<uint16_t*>(smem + PROF_BYTES);
   uint32_t* s_tab = reinterpret_cast<uint32_t*>(smem + PROF_BYTES + ROWOFF_BYTES);
-  uint8_t* s_ref = smem + p16_smem_fixed<G>();
+  uint8_t* s_ref = smem + P16_SMEM_FIXED;
 
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
-  const int sub = lane & (G - 1);                    // lane within the pair's group
-  const int hw = lane / G;                           // which pair of the warp
-  const unsigned gmask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (hw * G));
+  const int sub = lane & (P16_G - 1);                // lane within the pair's group
+  const int hw = lane / P16_G;                       // which pair of the warp
+  const unsigned gmask = 0xffffu << (hw * P16_G);
 
   if (p.ref_in_smem) {
     if (tid == 0) {
@@ -268,9 +257,9 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
   if (p.ref_in_smem) mbar_wait(&ref_bar, 0);
   __syncthreads();
 
-  uint16_t* rowA = s_rowoff + ((warp * NP + hw) * 2 + 0) * P16_MAXL;
-  uint16_t* rowB = s_rowoff + ((warp * NP + hw) * 2 + 1) * P16_MAXL;
-  uint32_t* tab = s_tab + (warp * NP + hw) * 2 * P16_TAB_WORDS;     // two buffers of P16_TAB_WORDS
+  uint16_t* rowA = s_rowoff + ((warp * P16_NP + hw) * 2 + 0) * P16_MAXL;
+  uint16_t* rowB = s_rowoff + ((warp * P16_NP + hw) * 2 + 1) * P16_MAXL;
+  uint32_t* tab = s_tab + (warp * P16_NP + hw) * 2 * P16_TAB_WORDS;     // two buffers of P16_TAB_WORDS
   const uint32_t prof_base = smem_u32(s_prof);
   const uint32_t tab_addr = smem_u32(tab);
 
@@ -288,11 +277,11 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
   const uint32_t rb_d2 = RB ? K2(p.rb_d) : 0u;
   uint32_t cur_n = 0;
 
-  // table entries this lane builds every row: e = sub + G*t -> (a, b) = (e / 5, e % 5)
+  // table entries this lane builds every row: e = sub + P16_G*t -> (a, b) = (e / 5, e % 5)
   uint32_t eoa[NE], eob[NE];
 #pragma unroll
   for (int t = 0; t < NE; t++) {
-    const int e = min(sub + G * t, 24);
+    const int e = min(sub + P16_G * t, 24);
     eoa[t] = (e / 5) * 2;
     eob[t] = (e % 5) * 2;
   }
@@ -301,7 +290,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
 #pragma unroll
     for (int t = 0; t < NE; t++) {
       const uint2 v = make_uint2((uint32_t)lds_s16(pa + eoa[t]), lds_u16(pb + eob[t]) << 16);
-      if (sub + G * t < 25) reinterpret_cast<uint2*>(dst)[sub + G * t] = v;
+      if (sub + P16_G * t < 25) reinterpret_cast<uint2*>(dst)[sub + P16_G * t] = v;
     }
   };
 
@@ -310,10 +299,10 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
     if (lane == 0) item = atomicAdd(p.counter, 1);
     item = __shfl_sync(0xffffffffu, item, 0);
     if (item >= n_items) break;
-    int rdA = p.pairs[2 * (item * NP + hw)];
-    int rdB = p.pairs[2 * (item * NP + hw) + 1];
+    int rdA = p.pairs[2 * (item * P16_NP + hw)];
+    int rdB = p.pairs[2 * (item * P16_NP + hw) + 1];
     const bool hasA = rdA >= 0;                       // an empty pair slot recomputes the warp's first pair and writes nothing
-    if (!hasA) rdA = p.pairs[2 * (item * NP)];
+    if (!hasA) rdA = p.pairs[2 * (item * P16_NP)];
     const bool hasB = hasA && rdB >= 0;
     if (rdB < 0 || !hasA) rdB = rdA;
     const int jrA = JOB ? p.job_read[rdA] : 0, jrB = JOB ? p.job_read[rdB] : 0;
@@ -338,7 +327,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
     if (RB) { cur_n = ((uint32_t)(-(GOP + 3 * GEP) - OFF + 32768) & 0xffffu) * 0x10001u; rb_ncmp0(); }
 
     __syncwarp();
-    for (int r = sub; r < L; r += G) {
+    for (int r = sub; r < L; r += P16_G) {
       const int d = sm_depth(r, L);
       rowA[r] = (uint16_t)(prof_row_index(sA, d, base_code(p.bases[oA + r])) * 2);
       rowB[r] = (uint16_t)(prof_row_index(sB, d, base_code(p.bases[oB + r])) * 2);
@@ -373,33 +362,15 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
 
     // Exclusive prefix over the group's lanes of the lane totals X (each in its own lane's frame): q of lane i = max over the lanes
     // l < i of X_l - CONV * (i - l), clamped so that nothing wraps (a clamped value ends at the bottom of the range, below every
-    // start-new level).  P16_SCAN4 = 0: four doubling steps + the shift by one lane = five dependent shuffles.  P16_SCAN4 = 1
-    // (16 lanes): the shift first, then windows of four lanes (three independent shuffles) and four windows (three more): three
-    // dependent shuffle latencies instead of five for six more instructions per row.  The scan's shuffles are where a warp waits
-    // (profiles/r02j_ncu_pair16_full.md: 28 % of the not-issued samples sit on the instruction behind each of them), yet the
-    // shorter chain measures SLOWER (K = 11: 1.365 -> 1.384 ms, K = 10: 1.156 -> 1.170 ms; bit-identical results): the other
-    // warps fill those waits already, what counts is the number of ALU-pipe instructions.  Kept as an option, off.
+    // start-new level): four doubling steps + the shift by one lane.
     auto lane_prefix = [&](uint32_t X) -> uint32_t {
-      if (P16_SCAN4 && G == 16) {
-        uint32_t s = __shfl_up_sync(0xffffffffu, X, 1, G);
-        s = __vadd2(__vmaxu2(s, B2(-32768 + CONV)), K2(-CONV)) & keep;          // s_i = X_(i-1) in lane i's frame; the first lane: bottom
-        const uint32_t a1 = __shfl_up_sync(0xffffffffu, s, 1, G), a2 = __shfl_up_sync(0xffffffffu, s, 2, G), a3 = __shfl_up_sync(0xffffffffu, s, 3, G);
-        uint32_t w = __viaddmax_u16x2(__vmaxu2(a1, B2(-32768 + CONV)), K2(-CONV), s);    // lanes < d get their own s back: max(s, max(s,cl)-dec) = s
-        w = __viaddmax_u16x2(__vmaxu2(a2, B2(-32768 + 2 * CONV)), K2(-2 * CONV), w);
-        w = __viaddmax_u16x2(__vmaxu2(a3, B2(-32768 + 3 * CONV)), K2(-3 * CONV), w);     // w_i covers s_(i-3) .. s_i
-        const uint32_t b1 = __shfl_up_sync(0xffffffffu, w, 4, G), b2 = __shfl_up_sync(0xffffffffu, w, 8, G), b3 = __shfl_up_sync(0xffffffffu, w, 12, G);
-        uint32_t q = __viaddmax_u16x2(__vmaxu2(b1, B2(-32768 + 4 * CONV)), K2(-4 * CONV), w);
-        q = __viaddmax_u16x2(__vmaxu2(b2, B2(-32768 + 8 * CONV)), K2(-8 * CONV), q);
-        q = __viaddmax_u16x2(__vmaxu2(b3, B2(-32768 + 12 * CONV)), K2(-12 * CONV), q);
-        return q;
-      }
       // inclusive cross-lane scan, converting by CONV per lane, clamped so nothing wraps
 #pragma unroll
-      for (int d = 1; d < G; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, X, d, G);
+      for (int d = 1; d < P16_G; d <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, X, d, P16_G);
         X = __viaddmax_u16x2(__vmaxu2(y, B2(-32768 + CONV * d)), K2(-CONV * d), X);    // lanes < d get their own X back: max(X, max(X,cl)-dec) = X
       }
-      const uint32_t q = __shfl_up_sync(0xffffffffu, X, 1, G);
+      const uint32_t q = __shfl_up_sync(0xffffffffu, X, 1, P16_G);
       return __vadd2(__vmaxu2(q, B2(-32768 + CONV)), K2(-CONV)) & keep;         // B2(-32768) = 0
     };
     // One DP row: row r-1 in W / acc -> row r in Wn / accn (Rg in place).  PAR = r & 1 selects the table buffer at
@@ -408,9 +379,9 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
     auto dp_row = [&](int r, auto par, const uint32_t (&W)[K], const uint32_t (&acc)[K], uint32_t (&Wn)[K], uint32_t (&accn)[K]) {
       constexpr int PAR = decltype(par)::value;
       if (r + 1 < L) build_table(r + 1, tab + (PAR ^ 1) * P16_TAB_WORDS);
-      uint32_t l2 = __shfl_up_sync(0xffffffffu, W[K - 2], 1, G);
-      uint32_t l1 = __shfl_up_sync(0xffffffffu, W[K - 1], 1, G);
-      uint32_t ain = __shfl_up_sync(0xffffffffu, acc[K - 1], 1, G);
+      uint32_t l2 = __shfl_up_sync(0xffffffffu, W[K - 2], 1, P16_G);
+      uint32_t l1 = __shfl_up_sync(0xffffffffu, W[K - 1], 1, P16_G);
+      uint32_t ain = __shfl_up_sync(0xffffffffu, acc[K - 1], 1, P16_G);
       l2 = and_or(__vadd2(l2, K2(-CONV)), keep, sentm);          // first lane of the group: no left neighbour
       const uint32_t l1c = __vadd2(l1, K2(-CONV));
       l1 = and_or(l1c, keep, sentm);
@@ -455,63 +426,17 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= P16_S
       rb_shift += p.rb_d;
       rb_ncmp0();
     };
-    // The same row, updated IN PLACE (G = 8: twice the columns per lane, no room for a second register set): the column-gap
-    // chain and the diagonal operand read row r-1's cells just before they are overwritten, two rotating registers deep.
-    auto dp_row_inplace = [&](int r, auto par, uint32_t (&W)[K], uint32_t (&acc)[K]) {
-      constexpr int PAR = decltype(par)::value;
-      if (r + 1 < L) build_table(r + 1, tab + (PAR ^ 1) * P16_TAB_WORDS);
-      uint32_t l2 = __shfl_up_sync(0xffffffffu, W[K - 2], 1, G);
-      uint32_t l1 = __shfl_up_sync(0xffffffffu, W[K - 1], 1, G);
-      uint32_t ain = __shfl_up_sync(0xffffffffu, acc[K - 1], 1, G);
-      l2 = and_or(__vadd2(l2, K2(-CONV)), keep, sentm);
-      const uint32_t l1c = __vadd2(l1, K2(-CONV));
-      l1 = and_or(l1c, keep, sentm);
-      ain &= keep;
-      uint32_t X = __vimax3_u16x2(l2, l1, W[0]);
+    uint32_t W1[K], acc1[K];
+    int r = 1;
+    for (; r + 1 < L; r += 2) {
+      if (RB && (r & (P16_RB_ROWS - 1)) == 1 && r > 1) rebase(W);
+      dp_row(r, std::integral_constant<int, 1>{}, W, acc, W1, acc1);
+      dp_row(r + 1, std::integral_constant<int, 0>{}, W1, acc1, W, acc);
+    }
+    if (r < L) {
+      dp_row(r, std::integral_constant<int, 1>{}, W, acc, W1, acc1);
 #pragma unroll
-      for (int j = 1; j + 1 < K - 2; j += 2) X = __vimax3_u16x2(X, W[j], W[j + 1]);
-      if ((K - 3) & 1) X = __vmaxu2(X, W[K - 3]);
-      X = __vadd2(X, K2(-GOP));
-      uint32_t q = lane_prefix(X);
-      uint32_t o2 = l2, o1 = l1, oa = ain;            // row r-1: cells j-2, j-1 and the verdict carry of cell j-1
-#pragma unroll
-      for (int j = 0; j < K; j++) {
-        const uint32_t ncmpj = B2(-(GOP + 3 * GEP) - OFF) + K2(GEP * j);
-        q = __viaddmax_u16x2(o2, K2(-GOP), q);        // Q[j]: max over columns <= c-2 of V - GOP
-        const uint32_t D = j > 0 ? o1 : and_or(l1c, keep, ncmp0m);
-        const uint32_t ad = oa;
-        const uint32_t best = __vimax3_u16x2(D, q, Rg[j]);
-        Rg[j] = __viaddmax_u16x2(D, K2(-GOP), Rg[j]);
-        const uint2 e = lds_entry<PAR * P16_TAB_WORDS * 4>(comb[j]);
-        uint32_t bp;
-        const uint32_t wn = cell_pair(best, ncmpj, e.x, e.y, gep2, bp);
-        const uint32_t an = (JOB && j == 0) ? and_or(bp ^ D, keep, ad) : (ad | (bp ^ D));
-        o2 = j > 0 ? o1 : l1;                         // row r-1's cell j-1 (the converted neighbour for j = 0)
-        o1 = W[j]; oa = acc[j];
-        W[j] = wn; acc[j] = an;
-      }
-      __syncwarp();
-    };
-    if (G == 8 || (P16_INPLACE && !JOB)) {
-      int r = 1;
-      for (; r + 1 < L; r += 2) {
-        dp_row_inplace(r, std::integral_constant<int, 1>{}, W, acc);
-        dp_row_inplace(r + 1, std::integral_constant<int, 0>{}, W, acc);
-      }
-      if (r < L) dp_row_inplace(r, std::integral_constant<int, 1>{}, W, acc);
-    } else {
-      uint32_t W1[K], acc1[K];
-      int r = 1;
-      for (; r + 1 < L; r += 2) {
-        if (RB && (r & (P16_RB_ROWS - 1)) == 1 && r > 1) rebase(W);
-        dp_row(r, std::integral_constant<int, 1>{}, W, acc, W1, acc1);
-        dp_row(r + 1, std::integral_constant<int, 0>{}, W1, acc1, W, acc);
-      }
-      if (r < L) {
-        dp_row(r, std::integral_constant<int, 1>{}, W, acc, W1, acc1);
-#pragma unroll
-        for (int j = 0; j < K; j++) { W[j] = W1[j]; acc[j] = acc1[j]; }
-      }
+      for (int j = 0; j < K; j++) { W[j] = W1[j]; acc[j] = acc1[j]; }
     }
 
     // ---- max_sg_score (first maximum of the last row) + the diagonal verdict, one read (half) at a time

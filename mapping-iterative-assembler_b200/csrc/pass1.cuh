@@ -19,7 +19,7 @@
 //                    frame; a read whose strands with hits are all jobs goes to the pair kernels, a read without hits
 //                    is skipped (mia_main.c:781), everything else (close stretches, saturated strand, long read)
 //                    goes to the general kernel (strip.cuh)
-//   pair16_kernel<K, G, true>   the jobs, two per register
+//   pair16_kernel<K, true>      the jobs, two per register
 //   p1_merge_kernel  first best job per strand, strand pick (forward only if strictly better, mia.c:1549-1554),
 //                    sg_align's coordinates (c2rcc, as / ae / start / end fix-ups, mia.c:1568-1610), or hand-over to
 //                    the general kernel when the winning job's alignment was not one plain diagonal

@@ -72,23 +72,6 @@ def test_iterate_host_equals_separate_calls(gpu):
         assert (out2[k] == out[k]).all(), k
 
 
-def test_pair16_eight_lane_variant_equals_default(gpu, monkeypatch):
-    # MIAGPU_PAIR_G=8: four pairs per warp, 16-22 columns per lane, rows updated in place -- same results, field for field
-    ref, bases, off, rc, as_, ae = gpu_checks.make_case(30000, 6000, seed=91, divergence=0.02, indel_rate=0.003, min_len=30, max_len=100)
-    gpu.set_pssm(gpu_checks.load_pssm("onepass"))
-    gpu.set_reference(ref, circular=1, with_rc=0)
-    a = gpu.realign_host(bases, off, rc, as_, ae)
-    monkeypatch.setenv("MIAGPU_PAIR_G", "8")
-    z = gpu.realign_host(bases, off, rc, as_, ae)
-    pb, _, _ = gpu.last_pair_buckets()
-    assert any(b["K"] >= 16 and b["reads"] > 1000 for b in pb), pb
-    for k in ("score", "as_out", "ae_out", "abr", "n_runs", "status"):
-        assert (np.asarray(a[k]) == np.asarray(z[k])).all(), k
-    nr = np.maximum(a["n_runs"], 0)
-    m = np.arange(a["runs"].shape[1])[None, :] < nr[:, None]
-    assert (np.where(m, a["runs"], 0) == np.where(m, z["runs"], 0)).all()
-
-
 @pytest.mark.parametrize("matrix,div,indel", [("pe", 0.01, 0.001), ("onepass", 0.12, 0.006), ("ancient", 0.30, 0.01)])
 def test_pair16_rebased_frame_takes_long_reads(gpu, monkeypatch, matrix, div, indel):
     # reads of 100-156 bases are beyond the low 16-bit frame (~130 rows): the RB variant (pair16.cuh 5.) takes them -- exact against the

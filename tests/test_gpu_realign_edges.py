@@ -1,9 +1,9 @@
 """-m gpu: a round's per-read realign against the oracle on every route classify_kernel can send a read down, read by read
 (score, as, ae, abr and both gapped strings).  Nothing here is compared with another GPU configuration.
 
-The routes: the eight 16-bit pair classes (128 ... 256 columns) in the low and the re-based (RB) frame, their MIAGPU_PAIR_G=8
-variants, the nine realign_kernel<K> buckets (<= 64 ... <= 512 columns), and the chunked strip kernels (team and warp) for
-windows over 512 columns and the whole-reference fallback (rs + L > re).  A read the pair kernels cannot finish is handed to a
+The routes: the eight 16-bit pair classes (128 ... 256 columns) in the low and the re-based (RB) frame, the nine
+realign_kernel<K> buckets (<= 64 ... <= 512 columns), and the chunked strip kernels (team and warp) for windows over 512
+columns and the whole-reference fallback (rs + L > re).  A read the pair kernels cannot finish is handed to a
 32-bit bucket with its window cut at its end cell; the cases below make that window land in bucket 0 and come out narrower
 than the read.
 
@@ -11,7 +11,8 @@ The case generator places every read so that the window rule of reiterate_assemb
 in the middle of the reference (ae - as = width - 100), at both clamps (as < 50, ae + 51 > wrap_len), across the end of a
 circular reference into its 256-base wrap copy, and beyond the window (the whole-reference fallback).  The widths are every
 edge E of the pair classes and the buckets at E and E + 1; the lengths 1, 2, 255, 256, the window's own width and the longest
-read of every pair class's low 16-bit frame and one more (pair16.cuh p16_lmax, which moves with the matrix's maximum).  The
+read of every pair class's low 16-bit frame and one more (pair16.cuh p16_lmax, which moves with the matrix's maximum), and the
+same at twice the columns per lane for the classes up to 176 columns (lengths just below those limits).  The
 contents: exact copies, substitutions, indels, insertions at the window's start, unrelated reads, low-complexity stretches
 (many tied end cells), N in the read and in the reference, and reads with 10 to 13 gaps around the 24-run limit.
 
@@ -29,13 +30,13 @@ pytestmark = pytest.mark.gpu
 GOP, GEP, PSSM_ABS_LIMIT, MAX_READ, MAX_RUNS, BUFFER = 1000, 200, 2000, 256, 24, 50
 ST_RUNS_OVERFLOW = 1
 P16_COLS = (128, 144, 160, 176, 192, 208, 224, 256)
-P16_G8 = (8, 8, 8, 8, 16, 16, 16, 16)                  # lanes per pair of every class under MIAGPU_PAIR_G=8
+NEAR_LIMIT_K = (16, 18, 20, 22, 12, 13, 14, 16)        # per pair class: the columns per lane of a second, lower length limit
 BUCKET_EDGES = (64, 128, 160, 192, 224, 256, 320, 384, 512)
 EDGES = sorted(set(P16_COLS) | set(BUCKET_EDGES))
 WIDTHS = sorted({w for e in EDGES for w in (e, e + 1)} | {1000})
 MATRICES = ("onepass", "ancient", "pe", "flat")
 KINDS = ("exact", "sub", "indel", "ins_head", "random", "lowcx", "nread", "nref")
-CONFIGS = {"default": {}, "pair16_off": {"MIAGPU_PAIR16": "0"}, "rb_off": {"MIAGPU_PAIR_RB": "0"}, "g8": {"MIAGPU_PAIR_G": "8"},
+CONFIGS = {"default": {}, "pair16_off": {"MIAGPU_PAIR16": "0"}, "rb_off": {"MIAGPU_PAIR_RB": "0"},
            "no_narrow": {"MIAGPU_NO_NARROW": "1"}, "strip_warp": {"MIAGPU_STRIP_TEAM": "0"}, "strip_team": {"MIAGPU_STRIP_TEAM": "1"}}
 ENV_KEYS = sorted({k for c in CONFIGS.values() for k in c} | {"MIAGPU_CHUNKS"})
 
@@ -48,9 +49,9 @@ def p16_lmax(K, max_entry):
 
 
 def low_frame_limits(sm):
-    """per pair class: the low frame's longest read with 16 and with MIAGPU_PAIR_G=8 lanes per pair"""
+    """per pair class: the low frame's longest read, and the same at NEAR_LIMIT_K columns per lane"""
     mx = int(np.max(sm))
-    return [(min(p16_lmax(c // 16, mx), MAX_READ), min(p16_lmax(c // g, mx), MAX_READ)) for c, g in zip(P16_COLS, P16_G8)]
+    return [(min(p16_lmax(c // 16, mx), MAX_READ), min(p16_lmax(k, mx), MAX_READ)) for c, k in zip(P16_COLS, NEAR_LIMIT_K)]
 
 
 def window(as_, ae, L, W):
@@ -108,8 +109,8 @@ class Case:
         for w in WIDTHS:
             cls = next((k for k, c in enumerate(P16_COLS) if w <= c), None)
             lens = {1, 2, 255, 256, w, w - 1, rng.randint(3, 254)}
-            for lo16, lo8 in limits:
-                lens |= {lo16, lo16 + 1, lo8, lo8 + 1}
+            for lim, near in limits:
+                lens |= {lim, lim + 1, near, near + 1}
             lens = sorted(L for L in lens if 1 <= L <= min(w, MAX_READ))
             places = ["left", "right"] + (["middle"] + (["wrap"] if circular else []) if w >= 100 else [])
             for place in places:
