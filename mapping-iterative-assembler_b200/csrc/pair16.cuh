@@ -27,9 +27,13 @@
 //
 // 3. One table read per cell pair, adds on the FMA pipe.  The substitution scores of a DP row depend
 //    on the column only through the two reference codes (a of read A's window, b of read B's), so each
-//    group keeps a 25-entry table of 64-bit entries  tab[a*5+b] = { (int32) subA(r,a), subB(r,b) << 16 }
+//    group keeps a 25-entry table of 64-bit entries  tab[p16_tab_entry(a,b)] = { (int32) subA(r,a), subB(r,b) << 16 }
 //    for the current row in shared memory (double-buffered, built for row r+1 while row r is
-//    computed): one LDS.64 per cell pair.  Because the halves are biased-unsigned and never leave
+//    computed): one LDS.64 per cell pair.  The kernel is bound by the shared-memory data pipe (DESIGN 4.2), so
+//    the table is laid out for it: a 64-bit load is served per half-warp (= one group), and the sixteen
+//    A/C/G/T pairs sit in entries 0..15, i.e. on sixteen distinct bank pairs -- one wavefront whatever the
+//    columns hold, where a*5+b put 0/16, 1/17 and 2/18 on one bank pair (1.82 wavefronts on random
+//    columns).  The row offsets of both reads of a group share one 32-bit word.  Because the halves are biased-unsigned and never leave
 //    [0, 65535], plain 32-bit adds (IMAD, FMA pipe -- the 16x2 min/max unit is the busy one) add each
 //    half exactly: the sign extension of the low entry cancels its borrow.  The start-new rule
 //    "S = N, substitution score NOT added" (mia.c:910-915) is the predicate on those two adds; the
@@ -67,6 +71,24 @@ constexpr int P16_NKB_WIDE = 8;                     // classes reiterate_assembl
 constexpr int P16_TAB_WORDS = 64;                   // 25 64-bit entries, padded to 32
 constexpr int P16_G = 16;                           // lanes per pair (1. in the header)
 constexpr int P16_NP = 32 / P16_G;                  // pairs per warp = per work item
+
+// Entry of the reference codes (a, b) in a group's substitution table (3. in the header): the A/C/G/T pairs at a*4+b, then
+// the nine pairs with an N (code 4): (N, b) at 16+b, (a, N) at 21+a.  p16_tab_a / p16_tab_b invert it for the table build.
+__host__ __device__ constexpr int p16_tab_entry(int a, int b) { return a < 4 && b < 4 ? a * 4 + b : a == 4 ? 16 + b : 21 + a; }
+__host__ __device__ constexpr int p16_tab_a(int e) { return e < 16 ? e >> 2 : e < 21 ? 4 : e - 21; }
+__host__ __device__ constexpr int p16_tab_b(int e) { return e < 16 ? e & 3 : e < 21 ? e - 16 : 4; }
+constexpr bool p16_tab_bijective() {
+  for (int e = 0; e < 25; e++)
+    if (p16_tab_a(e) > 4 || p16_tab_b(e) > 4 || p16_tab_entry(p16_tab_a(e), p16_tab_b(e)) != e) return false;
+  return true;
+}
+static_assert(p16_tab_bijective(), "p16_tab_entry maps the 25 code pairs onto 0..24");
+// Code of a padding column (c >= the window's length; the last lanes of a group).  Exact whatever it is: dyn_prog's candidates
+// of a cell all come from lower columns (mia.c:838-871), so a padding column feeds only padding columns; the end-cell key and
+// the verdict (max_sg_score) skip c >= len1; and the frame's bounds (2. and 5. above) use only the matrix's extreme entries,
+// never a column's code, so no value wraps.  Code 0 keeps a padding column's entry among the sixteen of distinct bank pairs,
+// where code 4 would share a bank pair with one of them.
+constexpr int P16_PAD_CODE = 0;
 
 // OFF of the lane frame: the lowest intermediate, (lowest cell = -OFF-GOP-GEP+min entry) converted to the next lane
 // (-GEP*K) minus GOP, must stay above -32768 for every matrix set_pssm accepts (|entry| <= PSSM_ABS_LIMIT).
@@ -211,8 +233,11 @@ __device__ __forceinline__ uint32_t cell_pair(uint32_t best, uint32_t ncmp, uint
   return w;
 }
 
-// dynamic shared memory: [prof16 (PROF16_N + 8) int16][rowoff WARPS*P16_NP*2*P16_MAXL u16][tab WARPS*P16_NP*2*P16_TAB_WORDS u32][ref codes]
-constexpr int P16_SMEM_FIXED = (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * P16_NP * 2 * P16_MAXL * 2 + WARPS_PER_BLOCK * P16_NP * 2 * P16_TAB_WORDS * 4;
+// dynamic shared memory: [prof16 (PROF16_N + 8) int16][rowoff WARPS*P16_MAXL*P16_NP u32][tab WARPS*P16_NP*2*P16_TAB_WORDS u32][ref codes]
+// rowoff: per warp, row r of pair hw in word r*P16_NP + hw = {shared address of read A's profile row, read B's << 16}: one LDS.32
+// per row, and the pairs of a warp, which run the same row, read adjacent banks.  The profile is the first section of the block's
+// shared memory (after at most a few bytes of static shared memory), so its addresses fit 16 bits.
+constexpr int P16_SMEM_FIXED = (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * P16_MAXL * P16_NP * 4 + WARPS_PER_BLOCK * P16_NP * 2 * P16_TAB_WORDS * 4;
 
 // JOB = false: a work item names reads (reiterate_assembly's windows, matrix by strand).
 // JOB = true : pass 1 with the k-mer filter (sg_align, mia.c:1500-1610).  A work item names jobs (pass1.cuh;
@@ -230,8 +255,8 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= 7 ? 6
   __shared__ __align__(8) uint64_t ref_bar;
   int16_t* s_prof = reinterpret_cast<int16_t*>(smem);
   constexpr int PROF_BYTES = (PROF16_N + 8) * 2;
-  constexpr int ROWOFF_BYTES = WARPS_PER_BLOCK * P16_NP * 2 * P16_MAXL * 2;
-  uint16_t* s_rowoff = reinterpret_cast<uint16_t*>(smem + PROF_BYTES);
+  constexpr int ROWOFF_BYTES = WARPS_PER_BLOCK * P16_MAXL * P16_NP * 4;
+  uint32_t* s_rowoff = reinterpret_cast<uint32_t*>(smem + PROF_BYTES);
   uint32_t* s_tab = reinterpret_cast<uint32_t*>(smem + PROF_BYTES + ROWOFF_BYTES);
   uint8_t* s_ref = smem + P16_SMEM_FIXED;
 
@@ -257,8 +282,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= 7 ? 6
   if (p.ref_in_smem) mbar_wait(&ref_bar, 0);
   __syncthreads();
 
-  uint16_t* rowA = s_rowoff + ((warp * P16_NP + hw) * 2 + 0) * P16_MAXL;
-  uint16_t* rowB = s_rowoff + ((warp * P16_NP + hw) * 2 + 1) * P16_MAXL;
+  uint32_t* rowAB = s_rowoff + warp * P16_MAXL * P16_NP + hw;          // row r: rowAB[r * P16_NP]
   uint32_t* tab = s_tab + (warp * P16_NP + hw) * 2 * P16_TAB_WORDS;     // two buffers of P16_TAB_WORDS
   const uint32_t prof_base = smem_u32(s_prof);
   const uint32_t tab_addr = smem_u32(tab);
@@ -277,16 +301,17 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= 7 ? 6
   const uint32_t rb_d2 = RB ? K2(p.rb_d) : 0u;
   uint32_t cur_n = 0;
 
-  // table entries this lane builds every row: e = sub + P16_G*t -> (a, b) = (e / 5, e % 5)
+  // table entries this lane builds every row: e = sub + P16_G*t -> (a, b) = (p16_tab_a(e), p16_tab_b(e))
   uint32_t eoa[NE], eob[NE];
 #pragma unroll
   for (int t = 0; t < NE; t++) {
     const int e = min(sub + P16_G * t, 24);
-    eoa[t] = (e / 5) * 2;
-    eob[t] = (e % 5) * 2;
+    eoa[t] = p16_tab_a(e) * 2;
+    eob[t] = p16_tab_b(e) * 2;
   }
   auto build_table = [&](int r, uint32_t* dst) {
-    const uint32_t pa = prof_base + rowA[r], pb = prof_base + rowB[r];
+    const uint32_t ab = rowAB[r * P16_NP];
+    const uint32_t pa = ab & 0xffffu, pb = ab >> 16;
 #pragma unroll
     for (int t = 0; t < NE; t++) {
       const uint2 v = make_uint2((uint32_t)lds_s16(pa + eoa[t]), lds_u16(pb + eob[t]) << 16);
@@ -329,17 +354,17 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, (K <= 5 ? 8 : K <= 7 ? 6
     __syncwarp();
     for (int r = sub; r < L; r += P16_G) {
       const int d = sm_depth(r, L);
-      rowA[r] = (uint16_t)(prof_row_index(sA, d, base_code(p.bases[oA + r])) * 2);
-      rowB[r] = (uint16_t)(prof_row_index(sB, d, base_code(p.bases[oB + r])) * 2);
+      rowAB[r * P16_NP] = (prof_base + prof_row_index(sA, d, base_code(p.bases[oA + r])) * 2) |
+                          (prof_base + prof_row_index(sB, d, base_code(p.bases[oB + r])) * 2) << 16;
     }
     uint32_t comb[K];                                 // shared address of the column's (a, b) entry in table buffer 0
 #pragma unroll
     for (int j = 0; j < K; j++) {
       const int c = sub * K + j;
-      int a = 4, b = 4;
+      int a = P16_PAD_CODE, b = P16_PAD_CODE;
       if (c < lenA) a = p.ref_in_smem ? s_ref[wsA + c] : p.ref_codes[wsA + c];
       if (c < lenB) b = p.ref_in_smem ? s_ref[wsB + c] : p.ref_codes[wsB + c];
-      comb[j] = tab_addr + (uint32_t)(a * 5 + b) * 8;
+      comb[j] = tab_addr + (uint32_t)p16_tab_entry(a, b) * 8;
     }
     __syncwarp();
     build_table(0, tab);

@@ -49,9 +49,11 @@ struct Sweep16Params {
   uint8_t* jstatus;
 };
 
-// dynamic shared memory: [prof16][rowoff WARPS*2*2*rows_cap u16][tab WARPS*2*2*P16_TAB_WORDS u32][ring WARPS*2*2*rows_cap*4 u32]
+// dynamic shared memory: [prof16][rowoff WARPS*rows_cap*2 u32][tab WARPS*2*2*P16_TAB_WORDS u32][ring WARPS*2*2*rows_cap*4 u32]
+// rowoff as in pair16.cuh: per warp, row r of half-warp hw in word r*2 + hw = {shared address of job A's profile row, job B's << 16}
+// (SAME: the one read's, whole word)
 __host__ __device__ constexpr int sw_smem(int rows_cap) {
-  return (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * 2 * 2 * rows_cap * 2 + WARPS_PER_BLOCK * 2 * 2 * P16_TAB_WORDS * 4 +
+  return (PROF16_N + 8) * 2 + WARPS_PER_BLOCK * rows_cap * 2 * 4 + WARPS_PER_BLOCK * 2 * 2 * P16_TAB_WORDS * 4 +
          WARPS_PER_BLOCK * 2 * 2 * rows_cap * 16;
 }
 
@@ -71,9 +73,9 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
   int16_t* s_prof = reinterpret_cast<int16_t*>(smem);
   constexpr int PROF_BYTES = (PROF16_N + 8) * 2;
   const int RC = p.rows_cap;                           // a multiple of 8: the sections stay 16-byte aligned
-  const int ROWOFF_BYTES = WARPS_PER_BLOCK * 2 * 2 * RC * 2;
+  const int ROWOFF_BYTES = WARPS_PER_BLOCK * RC * 2 * 4;
   constexpr int TAB_BYTES = WARPS_PER_BLOCK * 2 * 2 * P16_TAB_WORDS * 4;
-  uint16_t* s_rowoff = reinterpret_cast<uint16_t*>(smem + PROF_BYTES);
+  uint32_t* s_rowoff = reinterpret_cast<uint32_t*>(smem + PROF_BYTES);
   uint32_t* s_tab = reinterpret_cast<uint32_t*>(smem + PROF_BYTES + ROWOFF_BYTES);
   uint4* s_ring = reinterpret_cast<uint4*>(smem + PROF_BYTES + ROWOFF_BYTES + TAB_BYTES);
 
@@ -83,7 +85,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
   for (int i = tid; i < PROF16_N + 8; i += blockDim.x) s_prof[i] = p.prof16[i];
   __syncthreads();
 
-  uint16_t* rowA = s_rowoff + ((warp * 2 + hw) * 2 + 0) * RC;            // job B's rows: rowA + RC
+  uint32_t* rowAB = s_rowoff + warp * RC * 2 + hw;                     // row r: rowAB[2 * r]
   uint32_t* tab = s_tab + (warp * 2 + hw) * 2 * P16_TAB_WORDS;
   uint4* ring = s_ring + (size_t)(warp * 2 + hw) * 2 * RC;            // two buffers of RC rows: {l2, l1, acc, scan total}
   const uint32_t prof_base = smem_u32(s_prof);
@@ -104,12 +106,13 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
 #pragma unroll
   for (int t = 0; t < NE; t++) {
     const int e = min(sub + G * t, 24);
-    eoa[t] = (e / 5) * 2;
-    eob[t] = (e % 5) * 2;
+    eoa[t] = p16_tab_a(e) * 2;
+    eob[t] = p16_tab_b(e) * 2;
   }
-  // entry (a, b) = { sub_A(r, a), sub_B(r, b) << 16 }
+  // entry p16_tab_entry(a, b) = { sub_A(r, a), sub_B(r, b) << 16 }
   auto build_table = [&](int r, uint32_t* dst) {
-    const uint32_t pa = prof_base + rowA[r], pb = SAME ? pa : prof_base + rowA[RC + r];
+    const uint32_t ab = rowAB[2 * r];
+    const uint32_t pa = SAME ? ab : ab & 0xffffu, pb = SAME ? pa : ab >> 16;
 #pragma unroll
     for (int t = 0; t < NE; t++) {
       const uint2 v = make_uint2((uint32_t)lds_s16(pa + eoa[t]), lds_u16(pb + eob[t]) << 16);
@@ -131,7 +134,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
       const int64_t o = p.off[rd];
       L = (int)(p.off[rd + 1] - o);
       __syncwarp();
-      for (int r = sub; r < L; r += G) rowA[r] = (uint16_t)(prof_row_index(0, sm_depth(r, L), base_code(p.bases[o + r])) * 2);
+      for (int r = sub; r < L; r += G) rowAB[2 * r] = prof_base + prof_row_index(0, sm_depth(r, L), base_code(p.bases[o + r])) * 2;
       __syncwarp();
     } else {
       int jobA = p.pairs[4 * (int64_t)item + 2 * hw], jobB = p.pairs[4 * (int64_t)item + 2 * hw + 1];
@@ -146,8 +149,8 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
       __syncwarp();
       for (int r = sub; r < L; r += G) {
         const int d = sm_depth(r, L);
-        rowA[r] = (uint16_t)(prof_row_index(0, d, base_code(p.bases[oA + r])) * 2);
-        rowA[RC + r] = (uint16_t)(prof_row_index(0, d, base_code(p.bases[oB + r])) * 2);
+        rowAB[2 * r] = (prof_base + prof_row_index(0, d, base_code(p.bases[oA + r])) * 2) |
+                       (prof_base + prof_row_index(0, d, base_code(p.bases[oB + r])) * 2) << 16;
       }
       __syncwarp();
     }
@@ -170,12 +173,12 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4) sweep16_kernel(Sweep1
 #pragma unroll
       for (int j = 0; j < K; j++) {
         const int c = c0 + sub * K + j;
-        int a = 4, b = 4;
+        int a = P16_PAD_CODE, b = P16_PAD_CODE;      // padding columns: see P16_PAD_CODE (pair16.cuh)
         if (c < len1) {
           if (SAME) { a = __ldg(p.ref2 + c); b = __ldg(p.ref2 + p.strand_stride + c); }
           else { a = __ldg(p.ref2 + soA + c); b = __ldg(p.ref2 + soB + c); }
         }
-        comb[j] = tab_addr + (uint32_t)(a * 5 + b) * 8;
+        comb[j] = tab_addr + (uint32_t)p16_tab_entry(a, b) * 8;
       }
       __syncwarp();
       build_table(0, tab);
