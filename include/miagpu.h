@@ -425,8 +425,9 @@ int miagpu_shard_finish( miagpu_ctx* ctx, int cons_code, uint8_t* dropped,
  * *bytes = 0: no pointer state, nothing to do.  -D: miagpu_distant_retry_begin / _end before miagpu_shard_begin.  The repeat
  * filter is not available in sharded rounds. */
 int miagpu_shard_flags( miagpu_ctx* ctx, void** flag_buf, int64_t* bytes );
-/* chain blocks of the last round's regression that were summed read by read on the host, and how many of
- * those needed an extra device fetch (sharded rounds prefetch the likely ones with the block records) */
+/* chain blocks of the last round's regression that were summed read by read on the host.  A sharded round sends the
+ * keys of every block that cannot be proven with the block records, and a missing key is an error, so no block is
+ * ever fetched afterwards: *fetched_blocks is always 0. */
 int miagpu_last_cut_stats( miagpu_ctx* ctx, int64_t* serial_blocks, int64_t* fetched_blocks );
 
 /* Device-resident round (reads, rc, as, ae stay in HBM between calls): */

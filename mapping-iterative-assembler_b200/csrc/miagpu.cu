@@ -68,6 +68,16 @@ constexpr int MAX_DEVICES = 64;
 
 using namespace miagpu;
 
+// The score-cut policy of a whole round (miagpu_iterate_* or miagpu_shard_begin* .. _finish) and where its reads came from
+struct RoundPolicy {
+  int hard_cut = 0, score_cut_set = 0;          // -H, or a cut the caller gave (-S -N)
+  double slope = 0, intercept = 0;
+  bool unique_best = false;                     // the repeat filter's unique_best takes part in the cut
+  int host_chunks = 0;                          // > 0: the reads came from the host in that many chunks (host_round_front)
+  bool fit() const { return !score_cut_set && hard_cut <= 0; }
+  bool host_fed() const { return host_chunks > 0; }
+};
+
 struct miagpu_ctx {
   int device = 0;
   int num_sms = 0;
@@ -157,19 +167,15 @@ struct miagpu_ctx {
   DevBuf<uint64_t> rf_key, rf_key2;
   DevBuf<int64_t> rf_ord;
   DevBuf<int> rf_bad;
-  // sharded rounds (SURVEY 8e): this rank's part of the all-gather, what came back, prefetched chain blocks
-  int sh_world = 0, sh_rank = 0, sh_phase = 0, sh_hard_cut = 0, sh_cut_set = 0, sh_chunks = 0;
-  int64_t sh_nmax = 0, sh_stride = 0, sh_fetched = 0;
-  bool sh_fit = false, sh_host = false, sh_want_packed = false, sh_has_unique = false;
-  double sh_slope = 0, sh_icpt = 0;
-  DevBuf<uint32_t> d_sh_send, d_sh_recv, d_sh_pf;
+  RoundPolicy round;                            // the round in flight (one-GPU and sharded)
+  // sharded rounds (SURVEY 8e): this rank's part of the all-gather, what came back
+  int sh_world = 0, sh_rank = 0, sh_phase = 0;
+  int64_t sh_stride = 0;
+  DevBuf<uint32_t> d_sh_send, d_sh_recv;
   DevBuf<ShardPrep> d_sh_prep;
   int64_t sh_nb = 0;
   uint32_t* h_sh_recv = nullptr;                // pinned: what the all-gather of the block records brought
   size_t h_sh_cap = 0;
-  DevBuf<int32_t> d_sh_pfid;
-  uint32_t* h_sh_pf = nullptr;                  // pinned: SHARD_PF_SLOTS blocks of keys
-  int32_t* h_sh_pfid = nullptr;                 // pinned: count + block ids
   // pass 1 / wide windows
   int kmer_k = 0;
   DevBuf<int32_t> d_kb[2], d_kp[2];
@@ -324,9 +330,7 @@ extern "C" void miagpu_destroy(miagpu_ctx* c) {
   if (c->h_call) cudaFreeHost(c->h_call);
   if (c->h_sh_recv) cudaFreeHost(c->h_sh_recv);
   c->d_sh_prep.release();
-  if (c->h_sh_pf) cudaFreeHost(c->h_sh_pf);
-  if (c->h_sh_pfid) cudaFreeHost(c->h_sh_pfid);
-  c->d_sh_send.release(); c->d_sh_recv.release(); c->d_sh_pf.release(); c->d_sh_pfid.release();
+  c->d_sh_send.release(); c->d_sh_recv.release();
   c->tr_prof.release(); c->tr_ws.release(); c->tr_wl.release(); c->tr_out.release(); c->tr_cnt.release(); c->tr_codes.release();
   c->tr_ad.release(); c->tr_st.release();
   c->rf_rc.release(); c->rf_tr.release(); c->rf_uq.release(); c->rf_tmp.release(); c->rf_as.release(); c->rf_ae.release(); c->rf_k4.release();
@@ -1366,10 +1370,10 @@ static ConsParams cons_params(miagpu_ctx* c) {
 }
 
 // MODE 0 (per-position insert maxima) over the current entry list
-static int launch_gaps(miagpu_ctx* c) {
+static int launch_gaps(miagpu_ctx* c, cudaStream_t st) {
   if (!c->n_entries) return 1;
   ConsParams p = cons_params(c);
-  gaps_kernel<<<(unsigned)((c->n_entries + 255) / 256), 256, 0, c->stream>>>(p);          // a warp filters 32 entries
+  gaps_kernel<<<(unsigned)((c->n_entries + 255) / 256), 256, 0, st>>>(p);          // a warp filters 32 entries
   MIAGPU_CUDA(cudaGetLastError());
   c->launches++;
   return 1;
@@ -1387,15 +1391,14 @@ __global__ void to_host_kernel(uint32_t* __restrict__ dst, const uint32_t* __res
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < words; i += (int64_t)gridDim.x * blockDim.x) dst[i] = src[i];
 }
 static cudaError_t small_to_host(void* host_pinned, const void* dev, size_t bytes, cudaStream_t st) {
-  static const bool off = getenv("MIAGPU_NO_MAPPED_RESULTS") != nullptr;
-  if (off || ((uintptr_t)host_pinned & 3) || ((uintptr_t)dev & 3)) return cudaMemcpyAsync(host_pinned, dev, bytes, cudaMemcpyDeviceToHost, st);
+  if (((uintptr_t)host_pinned & 3) || ((uintptr_t)dev & 3)) return cudaMemcpyAsync(host_pinned, dev, bytes, cudaMemcpyDeviceToHost, st);
   const int64_t words = (int64_t)(bytes + 3) / 4;
   if (!words) return cudaSuccess;
   to_host_kernel<<<(unsigned)std::min<int64_t>(32, (words + 255) / 256), 256, 0, st>>>(static_cast<uint32_t*>(host_pinned), static_cast<const uint32_t*>(dev), words);
   return cudaGetLastError();
 }
 
-static int launch_accumulate(miagpu_ctx* c) {
+static int launch_accumulate(miagpu_ctx* c, cudaStream_t st) {
   if (!c->n_entries) return 1;
   ConsParams p = cons_params(c);
   const int n_tiles = (c->seq_len + TILE_POS - 1) / TILE_POS;
@@ -1407,19 +1410,19 @@ static int launch_accumulate(miagpu_ctx* c) {
     if (!c->d_ent_pos.reserve(9 * ne + 3 * MAX_TILES + 16)) return 0;
     TileRec* recs = reinterpret_cast<TileRec*>(c->d_ent_pos.p);
     int32_t *ent_tile = c->d_ent_pos.p + 8 * ne, *counts = ent_tile + ne, *starts = counts + MAX_TILES, *cursor = starts + MAX_TILES + 1;
-    MIAGPU_CUDA(cudaMemsetAsync(counts, 0, MAX_TILES * sizeof(int32_t), c->stream));
-    ent_bin_count_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, c->stream>>>(p, ent_tile, counts);
-    ent_bin_scan_kernel<<<1, 32, 0, c->stream>>>(n_tiles, counts, starts, cursor);
-    ent_bin_scatter_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, c->stream>>>(p, ent_tile, cursor, recs);
+    MIAGPU_CUDA(cudaMemsetAsync(counts, 0, MAX_TILES * sizeof(int32_t), st));
+    ent_bin_count_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(p, ent_tile, counts);
+    ent_bin_scan_kernel<<<1, 32, 0, st>>>(n_tiles, counts, starts, cursor);
+    ent_bin_scatter_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(p, ent_tile, cursor, recs);
     MIAGPU_CUDA(cudaGetLastError());
     const size_t smem = (size_t)TILE_SMEM_INTS * sizeof(int32_t);
     MIAGPU_CUDA(cudaFuncSetAttribute(tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int slices = std::max(1, (2 * c->num_sms + n_tiles - 1) / n_tiles);
-    tile_kernel<<<dim3(slices, n_tiles), TILE_THREADS, smem, c->stream>>>(p, recs, starts);
+    tile_kernel<<<dim3(slices, n_tiles), TILE_THREADS, smem, st>>>(p, recs, starts);
     MIAGPU_CUDA(cudaGetLastError());
     c->launches += 4;
   } else {
-    entry_kernel<1><<<(unsigned)((c->n_entries * 32 + 255) / 256), 256, 0, c->stream>>>(p);
+    entry_kernel<1><<<(unsigned)((c->n_entries * 32 + 255) / 256), 256, 0, st>>>(p);
     MIAGPU_CUDA(cudaGetLastError());
     c->launches++;
   }
@@ -1446,7 +1449,7 @@ extern "C" int miagpu_accumulate_gaps(miagpu_ctx* c, int64_t n_entries, const mi
   MIAGPU_CUDA(cudaEventRecord(c->ev[1], c->stream));
   c->n_entries = n_entries;
   MIAGPU_CUDA(cudaMemsetAsync(c->d_gaps.p, 0, (c->seq_len + 2) * sizeof(int32_t), c->stream));
-  if (!launch_gaps(c)) return 0;
+  if (!launch_gaps(c, c->stream)) return 0;
   MIAGPU_CUDA(cudaEventRecord(c->ev[2], c->stream));
   MIAGPU_CUDA(cudaStreamSynchronize(c->stream));
   MIAGPU_CUDA(cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]));
@@ -1473,7 +1476,7 @@ extern "C" int miagpu_accumulate_counts(miagpu_ctx* c, void** dev_counts, int64_
   c->n_cols = (int64_t)c->seq_len + total_ins;
   if (!c->d_acc.reserve(c->n_cols * NPLANE) || !c->d_called.reserve(c->n_cols + 16)) return 0;
   MIAGPU_CUDA(cudaMemsetAsync(c->d_acc.p, 0, c->n_cols * NPLANE * sizeof(int32_t), c->stream));
-  if (!launch_accumulate(c)) return 0;
+  if (!launch_accumulate(c, c->stream)) return 0;
   c->launches++;                                     // the scan
   MIAGPU_CUDA(cudaEventRecord(c->ev[2], c->stream));
   MIAGPU_CUDA(cudaStreamSynchronize(c->stream));
@@ -1570,7 +1573,7 @@ extern "C" int miagpu_accumulate_gaps_natural(miagpu_ctx* c, const uint8_t* drop
         dropped_back ? c->d_dropb.p : nullptr, c->d_entries.p);
     MIAGPU_CUDA(cudaGetLastError());
     c->launches++;
-    if (!launch_gaps(c)) return 0;
+    if (!launch_gaps(c, c->stream)) return 0;
   }
   MIAGPU_CUDA(cudaEventRecord(c->ev[2], c->stream));
   MIAGPU_CUDA(cudaStreamSynchronize(c->stream));
@@ -2367,23 +2370,164 @@ static int cut_launch_stats(miagpu_ctx* c, int64_t lo, int64_t hi, bool has_uniq
   return 1;
 }
 
+// ---- the phases of a round, one copy each for the one-GPU round (iterate_tail) and the sharded round (miagpu_shard_*).  The policy
+// is c->round.  Compute stream unless a phase takes one.
+
+// drains every stream a round puts work on: a round that fails leaves nothing of itself in flight
+static int round_abort(miagpu_ctx* c) {
+  if (c)
+    for (cudaStream_t st : {c->stream, c->s_up, c->s_down, c->s_aux[2]}) cudaStreamSynchronize(st);
+  return 0;
+}
+
+// a round over resident reads: pointer state (this round's results go to the partner buffers), integer sums zeroed, the DP (ev[1]..ev[2])
+static int round_start_resident(miagpu_ctx* c, bool sharded) {
+  if (c->fs_on) {
+    if (!fs_reserve_round(c)) return 0;
+    c->fs_sharded = sharded;
+    fs_begin_round(c);
+  }
+  MIAGPU_CUDA(cudaEventRecord(c->ev[1], c->stream));
+  cut_init_kernel<<<1, 256, 0, c->stream>>>(c->d_cstats.p);
+  MIAGPU_CUDA(cudaGetLastError());
+  if (!realign_device(c, false)) return 0;
+  MIAGPU_CUDA(cudaEventRecord(c->ev[2], c->stream));
+  return 1;
+}
+
+// entries (with the sticky flags of EARLIER rounds) + per-position insert maxima; none of it depends on this round's cut.  A host-fed
+// round's earlier flags arrive on the upload stream (xev[1]).
+static int round_entries(miagpu_ctx* c) {
+  cudaStream_t main = c->stream;
+  const int64_t n = c->n;
+  c->n_entries = 2 * n;
+  MIAGPU_CUDA(cudaMemsetAsync(c->d_gaps.p, 0, (c->seq_len + 2) * sizeof(int32_t), main));
+  if (c->round.host_fed()) MIAGPU_CUDA(cudaStreamWaitEvent(main, c->xev[1], 0));
+  if (c->fs_on) {
+    if (!fs_number_and_entries(c, c->round.unique_best)) return 0;
+  } else {
+    MIAGPU_CUDA(cudaMemsetAsync(c->d_fs_cnt.p, 0, FS_CNT_WORDS * sizeof(int32_t), main));
+    if (n) {
+      status_or_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_status.p, c->d_nruns.p, c->d_fs_cnt.p + FS_CNT_STATUS);
+      natural_entries_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_as_out.p, c->d_ae_out.p, c->d_nruns.p, c->d_runs.p,
+                                                                            c->d_status.p, c->seq_len, c->d_dropf.p, c->d_dropf.p, c->d_entries.p,
+                                                                            c->round.unique_best ? c->d_unique.p : nullptr);
+      MIAGPU_CUDA(cudaGetLastError());
+      c->launches += 2;
+    }
+  }
+  return launch_gaps(c, main);
+}
+
+// insert-column layout from the insert maxima; its total and the round's counters go to the host (aev[6])
+static int round_layout(miagpu_ctx* c) {
+  cudaStream_t main = c->stream;
+  CutHost* H = c->h_cut;
+  size_t tmp = 0;
+  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
+  if (!c->d_cub.reserve(tmp + 16)) return 0;
+  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
+  MIAGPU_CUDA(small_to_host(&H->total_ins, c->d_ins_off.p + c->seq_len, sizeof(int32_t), main));
+  MIAGPU_CUDA(small_to_host(H->fs_cnt, c->d_fs_cnt.p, sizeof(H->fs_cnt), main));
+  MIAGPU_CUDA(cudaEventRecord(c->aev[6], main));
+  c->launches += 2;
+  return 1;
+}
+
+// the column planes, sized on the host from the layout (one short wait) and zeroed on st; never a consensus that silently lacks reads
+static int round_planes(miagpu_ctx* c, cudaStream_t st) {
+  CutHost* H = c->h_cut;
+  MIAGPU_CUDA(cudaEventSynchronize(c->aev[6]));
+  if (c->fs_on) {
+    if (!fs_after_numbering(c, c->round.unique_best, H->fs_cnt, &H->total_ins)) return 0;
+  } else if (H->fs_cnt[FS_CNT_STATUS]) {
+    set_error("miagpu: reads came back with status bits 0x%x (more than %d alignment runs, or a window no kernel takes): the round is not usable", H->fs_cnt[FS_CNT_STATUS], MAX_RUNS);
+    return 0;
+  }
+  c->n_cols = (int64_t)c->seq_len + H->total_ins;
+  if (!c->d_acc.reserve(c->n_cols * NPLANE) || !c->d_called.reserve(c->n_cols + 16)) return 0;
+  MIAGPU_CUDA(cudaStreamWaitEvent(st, c->aev[6], 0));
+  MIAGPU_CUDA(cudaMemsetAsync(c->d_acc.p, 0, c->n_cols * NPLANE * sizeof(int32_t), st));
+  return 1;
+}
+
+// this round's flags (cull_maln_from_fsdb, mia.c:452-470), sticky (H10), and the newly dropped reads out of the base columns (xev[2]:
+// the flags are final).  Pointer state: through the pointers.  cut_first: the entries take this round's flags, then the one
+// accumulation.  Otherwise the columns were accumulated with the earlier flags and the newly dropped reads are taken back out.
+static int round_flags(miagpu_ctx* c, double slope, double intercept, bool cut_first) {
+  cudaStream_t main = c->stream;
+  const int64_t n = c->n;
+  CutHost* H = c->h_cut;
+  cut_thresholds(c->round.hard_cut, slope, intercept, H->thr);
+  MIAGPU_CUDA(cudaMemcpyAsync(c->d_thr.p, H->thr, sizeof(H->thr), cudaMemcpyHostToDevice, main));
+  if (n && c->fs_on) {
+    if (!fs_flags_and_undo(c, c->round.unique_best)) return 0;
+  } else if (n) {
+    cut_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_seqlen.p, c->d_score.p, c->d_thr.p, c->d_dropf.p, cut_first ? c->d_entries.p : nullptr,
+                                                                    c->d_cstats.p, c->round.unique_best ? c->d_unique.p : nullptr, c->d_newly.p);
+    MIAGPU_CUDA(cudaGetLastError());
+    c->launches++;
+    if (cut_first) {
+      if (!launch_accumulate(c, main)) return 0;
+    } else {
+      undo_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(cons_params(c), n, c->d_newly.p, c->d_entries.p);
+      MIAGPU_CUDA(cudaGetLastError());
+      c->launches++;
+    }
+  }
+  MIAGPU_CUDA(cudaEventRecord(c->xev[2], main));
+  return 1;
+}
+
+// base calling (consensus_assembly_string); the flags go to the host on the download stream meanwhile
+static int round_call(miagpu_ctx* c, int cons_code, uint8_t* dropped, int32_t* gaps_out, char* cons_out, int32_t* cons_len) {
+  if (dropped && c->n) {
+    MIAGPU_CUDA(cudaStreamWaitEvent(c->s_down, c->xev[2], 0));
+    MIAGPU_CUDA(cudaMemcpyAsync(dropped, c->d_dropf.p, c->n, cudaMemcpyDeviceToHost, c->s_down));   // fs mode: AlnSeq.dropped behind front_asp (fs_flags_and_undo)
+  }
+  c->cons_stage = 2;
+  const int launches = c->launches;
+  if (!miagpu_call(c, cons_code, gaps_out, nullptr, cons_out, cons_len)) return 0;
+  c->launches = launches + 1;
+  return 1;
+}
+
+// after base calling: the round's timing and fallback count; the device state is now that of a round that called its bases
+static int round_end(miagpu_ctx* c) {
+  if (c->round.host_fed()) {
+    c->ms_h2d = 0; c->ms_kernels = 0; c->ms_d2h = 0;   // the phases overlap: only the caller's wall clock means something
+    MIAGPU_CUDA(cudaStreamSynchronize(c->s_up));
+    for (int k = 0; k < c->round.host_chunks; k++) {
+      int32_t nf = 0;
+      MIAGPU_CUDA(cudaMemcpy(&nf, c->d_meta.p + (size_t)META_WORDS * k + META_NFALL, 4, cudaMemcpyDeviceToHost));
+      c->n_fallback += nf;
+    }
+  } else {
+    MIAGPU_CUDA(cudaEventElapsedTime(&c->ms_kernels, c->ev[1], c->ev[2]));
+    c->ms_h2d = c->ms_d2h = 0;
+    MIAGPU_CUDA(cudaMemcpy(&c->n_fallback, c->d_meta.p + META_NFALL, 4, cudaMemcpyDeviceToHost));
+    if (c->fs_on) c->fs_prev_seq_len = c->seq_len;   // the geometry of this round's alignments, should the next round have to freeze one
+  }
+  c->misinc_stale = nullptr;
+  return 1;
+}
+
 struct IterTail {
   // what the host knows about the reads (fallback blocks of the chains are summed on the host, read by read)
   const int32_t* h_seq_len; const uint8_t* h_unique; const int32_t* h_score; cudaEvent_t scores_on_host;
-  bool wait_old_flags;                               // c->xev[1]: the earlier rounds' flags are on the device
-  int hard_cut, score_cut_set; double slope, intercept; int cons_code;
+  int cons_code;
   // outputs (host, nullable)
   uint16_t* packed_runs; int64_t capacity; int64_t* total_runs; uint8_t* dropped; int32_t* gaps_out; char* cons_out; int32_t* cons_len;
   double* slope_out; double* intercept_out;
 };
 
-// Everything after the DP of one round: score cut (stats kernels already enqueued per chunk), entries, insert maxima,
+// Everything after the DP of a one-GPU round: score cut (stats kernels already enqueued per chunk), entries, insert maxima,
 // column accumulation, base calling.  Compute stream throughout; two short host waits (the integer sums, the blocks).
 static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
   cudaStream_t main = c->stream, down = c->s_down, side = c->s_aux[2];
   const int64_t n = c->n;
-  const bool fit = !a.score_cut_set && a.hard_cut <= 0;
-  const bool has_unique = a.h_unique != nullptr;
+  const bool fit = c->round.fit();
+  const bool has_unique = c->round.unique_best;
   CutHost* H = c->h_cut;
   const int64_t nb = (n + CUT_BLOCK - 1) / CUT_BLOCK;
   if (!c->d_newly.reserve(n + 1)) return 0;
@@ -2391,43 +2535,21 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
     MIAGPU_CUDA(small_to_host(&H->stats, c->d_cstats.p, sizeof(CutStatsDev), main));
     MIAGPU_CUDA(cudaEventRecord(c->xev[0], main));
   }
-  // ---- packed run lists + entries + per-position insert maxima: none of it depends on this round's cut.  The entries take
-  // the sticky flags of EARLIER rounds; the reads this round drops are taken back out of the planes afterwards (undo_kernel),
-  // so that the column accumulation runs while the host stitches the regression's chains.
+  // ---- packed run lists + entries + per-position insert maxima.  The reads this round drops are taken back out of the planes
+  // afterwards (round_flags), so that the column accumulation runs while the host stitches the regression's chains.
   int64_t* cnt = c->d_off2.p;
   int64_t* offs = c->d_off2.p + (n + 2);
-  size_t tmp = 0, tmp2 = 0;
-  const bool want_packed = a.packed_runs || a.total_runs;
-  if (want_packed) MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, offs, n + 1, main));
-  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp2, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
-  if (!c->d_cub.reserve(std::max(tmp, tmp2) + 16)) return 0;
   H->tot_runs = 0;
-  if (want_packed) {
+  if (a.packed_runs || a.total_runs) {
+    size_t tmp = 0;
+    MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, offs, n + 1, main));
+    if (!c->d_cub.reserve(tmp + 16)) return 0;
     clamp_runs_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, main>>>(n, c->d_nruns.p, cnt);
     MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp, cnt, offs, n + 1, main));
     MIAGPU_CUDA(small_to_host(&H->tot_runs, offs + n, 8, main));
     c->launches += 3;
   }
-  c->n_entries = 2 * n;
-  MIAGPU_CUDA(cudaMemsetAsync(c->d_gaps.p, 0, (c->seq_len + 2) * sizeof(int32_t), main));
-  if (a.wait_old_flags) MIAGPU_CUDA(cudaStreamWaitEvent(main, c->xev[1], 0));          // the earlier rounds' flags are on the device
-  if (c->fs_on) {
-    if (!fs_number_and_entries(c, has_unique)) return 0;
-  } else {
-    MIAGPU_CUDA(cudaMemsetAsync(c->d_fs_cnt.p, 0, FS_CNT_WORDS * sizeof(int32_t), main));
-    status_or_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_status.p, c->d_nruns.p, c->d_fs_cnt.p + FS_CNT_STATUS);
-    natural_entries_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_as_out.p, c->d_ae_out.p, c->d_nruns.p, c->d_runs.p,
-                                                                          c->d_status.p, c->seq_len, c->d_dropf.p, c->d_dropf.p, c->d_entries.p,
-                                                                          has_unique ? c->d_unique.p : nullptr);
-    MIAGPU_CUDA(cudaGetLastError());
-    c->launches += 2;
-  }
-  if (!launch_gaps(c)) return 0;
-  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp2, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
-  MIAGPU_CUDA(small_to_host(&H->total_ins, c->d_ins_off.p + c->seq_len, sizeof(int32_t), main));
-  MIAGPU_CUDA(small_to_host(H->fs_cnt, c->d_fs_cnt.p, sizeof(H->fs_cnt), main));
-  MIAGPU_CUDA(cudaEventRecord(c->aev[6], main));
-  c->launches += 2;
+  if (!round_entries(c) || !round_layout(c)) return 0;
   tr.mark("entries + insert maxima enqueued");
   // ---- regression: integer sums -> tables -> block kernels (side stream) -> stitch (find_fsdb_score_cut, fsdb.c:269-383)
   CutSums S;
@@ -2437,7 +2559,7 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
     tr.mark("integer sums on host");
     S.sx = H->stats.sx; S.sy = H->stats.sy; S.cnt = H->stats.cnt; S.bad = H->stats.bad == LLONG_MAX ? -1 : H->stats.bad;
     memcpy(S.best, H->stats.best, sizeof(S.best));
-    if (S.bad >= 0) { cudaStreamSynchronize(main); set_error("miagpu_score_cut: seq_len[%lld] = %d out of range", (long long)S.bad, a.h_seq_len[S.bad]); return 0; }
+    if (S.bad >= 0) { set_error("miagpu_score_cut: seq_len[%lld] = %d out of range", (long long)S.bad, a.h_seq_len[S.bad]); return 0; }
     cut_fit_tables(S, F);
     H->tab.ybar = F.ybar;
     memcpy(H->tab.dx, F.dx_of, sizeof(F.dx_of));
@@ -2456,27 +2578,18 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
     c->launches += 2;
   }
   // ---- column accumulation of every read that is not yet dropped (needs the insert-column layout: one short wait)
-  MIAGPU_CUDA(cudaEventSynchronize(c->aev[6]));
-  if (c->fs_on && !fs_after_numbering(c, has_unique, H->fs_cnt, &H->total_ins)) { cudaStreamSynchronize(main); cudaStreamSynchronize(side); return 0; }
-  if (!c->fs_on && H->fs_cnt[FS_CNT_STATUS]) {       // never a consensus that silently lacks reads
-    cudaStreamSynchronize(main); cudaStreamSynchronize(side);
-    set_error("miagpu: reads came back with status bits 0x%x (more than %d alignment runs, or a window no kernel takes): the round is not usable", H->fs_cnt[FS_CNT_STATUS], MAX_RUNS);
-    return 0;
-  }
+  if (!round_planes(c, main)) return 0;
   const int64_t tot = H->tot_runs;
   if (a.total_runs) *a.total_runs = tot;
-  if (a.packed_runs && tot > a.capacity) { cudaStreamSynchronize(main); cudaStreamSynchronize(side); set_error("miagpu_iterate: %lld runs, capacity %lld", (long long)tot, (long long)a.capacity); return 0; }
+  if (a.packed_runs && tot > a.capacity) { set_error("miagpu_iterate: %lld runs, capacity %lld", (long long)tot, (long long)a.capacity); return 0; }
   if (!c->d_packed.reserve(tot + 1)) return 0;
-  c->n_cols = (int64_t)c->seq_len + H->total_ins;
-  if (!c->d_acc.reserve(c->n_cols * NPLANE) || !c->d_called.reserve(c->n_cols + 16)) return 0;
-  MIAGPU_CUDA(cudaMemsetAsync(c->d_acc.p, 0, c->n_cols * NPLANE * sizeof(int32_t), main));
   // Normally the columns of every read not yet dropped are accumulated while the host stitches the chains, and the few reads this
   // round's cut drops are taken back out afterwards.  When the previous round dropped more than an eighth of the reads (the first
   // rounds on a divergent seed: mia.c:452-470 cuts most of them), the same is likely now: wait for the cut, flag the entries,
   // and accumulate once.  Integer sums: the planes are the same either way.
   // (a cut the caller gave -- -H / -S -N -- is known at once: flags first, always)
-  const bool cut_first = !c->fs_on && (!fit || (c->cut_prev_newly >= 0 && c->cut_prev_newly * 8 > n)) && !getenv("MIAGPU_NO_CUT_FIRST");
-  if (!cut_first && !launch_accumulate(c)) return 0;
+  const bool cut_first = !c->fs_on && (!fit || (c->cut_prev_newly >= 0 && c->cut_prev_newly * 8 > n));
+  if (!cut_first && !launch_accumulate(c, main)) return 0;
   if (a.packed_runs) {
     pack_runs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_nruns.p, offs, c->d_runs.p, c->d_packed.p);
     MIAGPU_CUDA(cudaEventRecord(c->xev[3], main));
@@ -2485,7 +2598,7 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
     c->launches++;
   }
   tr.mark("accumulation enqueued");
-  double slope = a.slope, intercept = a.intercept;
+  double slope = c->round.slope, intercept = c->round.intercept;
   if (fit) {
     MIAGPU_CUDA(cudaEventSynchronize(c->aev[7]));
     MIAGPU_CUDA(cudaEventSynchronize(a.scores_on_host));
@@ -2507,36 +2620,11 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
   }
   if (a.slope_out) *a.slope_out = slope;
   if (a.intercept_out) *a.intercept_out = intercept;
-  // ---- this round's flags (cull_maln_from_fsdb, mia.c:452-470), sticky (H10); the newly dropped reads leave the base columns
-  cut_thresholds(a.hard_cut, slope, intercept, H->thr);
-  MIAGPU_CUDA(cudaMemcpyAsync(c->d_thr.p, H->thr, sizeof(H->thr), cudaMemcpyHostToDevice, main));
-  if (c->fs_on) {
-    if (!fs_flags_and_undo(c, has_unique)) return 0;
-  } else if (cut_first) {                              // the entries take this round's flags, then one accumulation
-    cut_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_seqlen.p, c->d_score.p, c->d_thr.p, c->d_dropf.p, c->d_entries.p, c->d_cstats.p,
-                                                                    has_unique ? c->d_unique.p : nullptr, c->d_newly.p);
-    MIAGPU_CUDA(cudaGetLastError());
-    c->launches += 1;
-    if (!launch_accumulate(c)) return 0;
-  } else {
-    cut_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_seqlen.p, c->d_score.p, c->d_thr.p, c->d_dropf.p, nullptr, c->d_cstats.p,
-                                                                    has_unique ? c->d_unique.p : nullptr, c->d_newly.p);
-    undo_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(cons_params(c), n, c->d_newly.p, c->d_entries.p);
-    MIAGPU_CUDA(cudaGetLastError());
-    c->launches += 2;
-  }
+  if (!round_flags(c, slope, intercept, cut_first)) return 0;
   MIAGPU_CUDA(small_to_host(&H->newly_dropped, &c->d_cstats.p->pad, sizeof(int32_t), main));
   MIAGPU_CUDA(small_to_host(&H->bad_after, &c->d_cstats.p->bad, sizeof(long long), main));
-  MIAGPU_CUDA(cudaEventRecord(c->xev[2], main));
-  if (a.dropped) {
-    MIAGPU_CUDA(cudaStreamWaitEvent(down, c->xev[2], 0));
-    MIAGPU_CUDA(cudaMemcpyAsync(a.dropped, c->d_dropf.p, n, cudaMemcpyDeviceToHost, down));     // fs mode: AlnSeq.dropped behind front_asp (fs_flags_and_undo)
-  }
   tr.mark("flags + undo enqueued");
-  c->cons_stage = 2;
-  const int launches = c->launches;
-  if (!miagpu_call(c, a.cons_code, a.gaps_out, nullptr, a.cons_out, a.cons_len)) return 0;
-  c->launches = launches + 1;
+  if (!round_call(c, a.cons_code, a.dropped, a.gaps_out, a.cons_out, a.cons_len)) return 0;
   tr.mark("consensus called and downloaded");
   if (H->bad_after != LLONG_MAX) { set_error("miagpu_cull_flags: seq_len[%lld] = %d out of range", H->bad_after, a.h_seq_len[H->bad_after]); return 0; }
   c->cut_prev_newly = c->fs_on ? -1 : H->newly_dropped;
@@ -2557,11 +2645,11 @@ static int iterate_tail(miagpu_ctx* c, const IterTail& a, const Trace& tr) {
 //                   compute stream accumulates)
 //   download stream chunk k's scores (first) and the other per-read outputs while chunk k+1 computes
 // upload, per-chunk classification + DP + downloads of a host-resident batch (the front half of a round); returns the
-// number of chunks through *chunks (the last chunk's "scores on host" event is c->cev[4 * (C - 1) + 2])
+// number of chunks C, 0 on error (the last chunk's "scores on host" event is c->cev[4 * (C - 1) + 2])
 static int host_round_front(miagpu_ctx* c, const char* who, int64_t n, const uint8_t* bases, const int64_t* offsets, const uint8_t* rc,
                             const int32_t* as, const int32_t* ae, int32_t* score, int32_t* as_out, int32_t* ae_out, int32_t* abr,
                             int32_t* n_runs, uint8_t* status, const int32_t* seq_len, const uint8_t* unique_best, bool stats,
-                            const uint8_t* dropped, const Trace& tr, int* chunks) {
+                            const uint8_t* dropped, const Trace& tr) {
   if (!c || !c->have_pssm || !c->have_ref) { set_error("%s: set_pssm and set_reference first", who); return 0; }
   misinc_invalidate(c, "a new round has started and not ended");
   if (n <= 0 || !bases || !offsets || !rc || !as || !ae || !score || !seq_len || !dropped) { set_error("%s: bad argument", who); return 0; }
@@ -2575,7 +2663,6 @@ static int host_round_front(miagpu_ctx* c, const char* who, int64_t n, const uin
       !cut_reserve(c, n)) return 0;
   cudaStream_t main = c->stream, up = c->s_up, down = c->s_down;
   const int C = pick_chunks(n);
-  *chunks = C;
   tr.mark("buffers reserved");
   realign_reset_stats(c);
   c->n = n; c->total_bases = total; c->cut_inputs_n = -1;
@@ -2632,17 +2719,7 @@ static int host_round_front(miagpu_ctx* c, const char* who, int64_t n, const uin
     if (status) MIAGPU_CUDA(cudaMemcpyAsync(status + j.lo, c->d_status.p + j.lo, j.n, cudaMemcpyDeviceToHost, down));
   }
   tr.mark("DP + downloads enqueued");
-  return 1;
-}
-// the chunks' statistics after a round that went through host_round_front
-static int host_round_stats(miagpu_ctx* c, int C) {
-  c->ms_h2d = 0; c->ms_kernels = 0; c->ms_d2h = 0;   // the phases overlap: only the caller's wall clock means something
-  for (int k = 0; k < C; k++) {
-    int32_t nf = 0;
-    MIAGPU_CUDA(cudaMemcpy(&nf, c->d_meta.p + (size_t)META_WORDS * k + META_NFALL, 4, cudaMemcpyDeviceToHost));
-    c->n_fallback += nf;
-  }
-  return 1;
+  return C;
 }
 
 extern "C" int miagpu_iterate_host(miagpu_ctx* c, int64_t n, const uint8_t* bases, const int64_t* offsets, const uint8_t* rc,
@@ -2651,28 +2728,23 @@ extern "C" int miagpu_iterate_host(miagpu_ctx* c, int64_t n, const uint8_t* base
                                    int64_t* total_runs, const int32_t* seq_len, const uint8_t* unique_best, int hard_cut,
                                    int score_cut_set, double slope, double intercept, uint8_t* dropped, int cons_code,
                                    int32_t* gaps_out, char* cons_out, int32_t* cons_len) {
-  const bool fit = !score_cut_set && hard_cut <= 0;
   const Trace tr;
-  int C = 1;
-  if (!host_round_front(c, "miagpu_iterate_host", n, bases, offsets, rc, as, ae, score, as_out, ae_out, abr, n_runs, status, seq_len,
-                        unique_best, fit, dropped, tr, &C)) {
-    if (c && c->s_up) { cudaStreamSynchronize(c->s_down); cudaStreamSynchronize(c->s_up); }
-    return 0;
-  }
-  cudaStream_t down = c->s_down, up = c->s_up;
+  RoundPolicy pol{hard_cut, score_cut_set, slope, intercept, unique_best != nullptr};
+  const int C = host_round_front(c, "miagpu_iterate_host", n, bases, offsets, rc, as, ae, score, as_out, ae_out, abr, n_runs, status, seq_len,
+                                 unique_best, pol.fit(), dropped, tr);
+  if (!C) return round_abort(c);
+  pol.host_chunks = C;
+  c->round = pol;
   IterTail t{};
-  t.h_seq_len = seq_len; t.h_unique = unique_best; t.h_score = score; t.scores_on_host = c->cev[4 * (C - 1) + 2];
-  t.wait_old_flags = true;
-  t.hard_cut = hard_cut; t.score_cut_set = score_cut_set; t.slope = slope; t.intercept = intercept; t.cons_code = cons_code;
+  t.h_seq_len = seq_len; t.h_unique = unique_best; t.h_score = score; t.scores_on_host = c->cev[4 * (C - 1) + 2]; t.cons_code = cons_code;
   t.packed_runs = packed_runs; t.capacity = capacity; t.total_runs = total_runs; t.dropped = dropped;
   t.gaps_out = gaps_out; t.cons_out = cons_out; t.cons_len = cons_len;
-  if (!iterate_tail(c, t, tr)) { cudaStreamSynchronize(down); cudaStreamSynchronize(up); return 0; }
+  if (!iterate_tail(c, t, tr)) return round_abort(c);
   if (tr.on) {                                       // device time from the first chunk's DP launch to the last chunk's last DP kernel
     float ms = 0;
     if (cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]) == cudaSuccess) fprintf(stderr, "[miagpu trace] DP of %d chunk(s) on the device: %.3f ms\n", C, ms);
   }
-  if (!host_round_stats(c, C)) return 0;
-  c->misinc_stale = nullptr;
+  if (!round_end(c)) return round_abort(c);
   return 1;
 }
 
@@ -2719,41 +2791,24 @@ extern "C" int miagpu_iterate_resident(miagpu_ctx* c, int hard_cut, int score_cu
     MIAGPU_CUDA(cudaMallocHost(&c->h_score, sizeof(int32_t) * (n + 64)));
     c->h_score_cap = n;
   }
-  const bool fit = !score_cut_set && hard_cut <= 0;
+  c->round = RoundPolicy{hard_cut, score_cut_set, slope, intercept, !c->h_unique.empty()};
   const Trace tr;
-  cudaStream_t main = c->stream, down = c->s_down;
-  if (c->fs_on) {
-    if (!fs_reserve_round(c)) return 0;
-    c->fs_sharded = false;
-    fs_begin_round(c);
-  }
-  MIAGPU_CUDA(cudaEventRecord(c->ev[1], main));
-  cut_init_kernel<<<1, 256, 0, main>>>(c->d_cstats.p);
-  MIAGPU_CUDA(cudaGetLastError());
-  if (!realign_device(c, false)) return 0;
-  MIAGPU_CUDA(cudaEventRecord(c->ev[2], main));
-  if (fit) {
+  if (!round_start_resident(c, false)) return round_abort(c);
+  if (c->round.fit()) {
+    cudaStream_t down = c->s_down;
     MIAGPU_CUDA(cudaStreamWaitEvent(down, c->ev[2], 0));
     MIAGPU_CUDA(cudaMemcpyAsync(c->h_score, c->d_score.p, n * 4, cudaMemcpyDeviceToHost, down));    // only the chains' unproven blocks read them
     MIAGPU_CUDA(cudaEventRecord(c->cev[2], down));
-    if (!cut_launch_stats(c, 0, n, !c->h_unique.empty())) return 0;
+    if (!cut_launch_stats(c, 0, n, c->round.unique_best)) return round_abort(c);
   }
   tr.mark("DP enqueued");
   IterTail t{};
-  t.h_seq_len = c->h_seqlen.data(); t.h_unique = c->h_unique.empty() ? nullptr : c->h_unique.data(); t.h_score = c->h_score;
-  t.scores_on_host = c->cev[2]; t.wait_old_flags = false;
-  t.hard_cut = hard_cut; t.score_cut_set = score_cut_set; t.slope = slope; t.intercept = intercept; t.cons_code = cons_code;
+  t.h_seq_len = c->h_seqlen.data(); t.h_unique = c->round.unique_best ? c->h_unique.data() : nullptr; t.h_score = c->h_score;
+  t.scores_on_host = c->cev[2]; t.cons_code = cons_code;
   t.dropped = dropped; t.gaps_out = gaps_out; t.cons_out = cons_out; t.cons_len = cons_len;
   t.slope_out = slope_out; t.intercept_out = intercept_out;
-  if (!iterate_tail(c, t, tr)) { cudaStreamSynchronize(down); return 0; }
-  MIAGPU_CUDA(cudaEventElapsedTime(&c->ms_kernels, c->ev[1], c->ev[2]));
-  c->ms_h2d = c->ms_d2h = 0;
-  MIAGPU_CUDA(cudaMemcpy(&c->n_fallback, c->d_meta.p + META_NFALL, 4, cudaMemcpyDeviceToHost));
-  if (c->fs_on) {
-    c->fs_prev_seq_len = c->seq_len;                 // the geometry of this round's alignments, should the next round have to freeze one
-    fs_carry_submat(c);
-  }
-  c->misinc_stale = nullptr;
+  if (!iterate_tail(c, t, tr) || !round_end(c)) return round_abort(c);
+  if (c->fs_on) fs_carry_submat(c);
   return 1;
 }
 
@@ -2791,19 +2846,17 @@ static int shard_reserve(miagpu_ctx* c, int world, int64_t n_max) {
   return 1;
 }
 
-// after the DP: this rank's header row + insert maxima + best scores for the all-reduce(MAX), and the flag-independent part of the consensus
-static int shard_after_dp(miagpu_ctx* c, bool stats_done, bool has_unique, void** max_buf, int64_t* max_words) {
+// after the DP: this rank's entries and insert maxima, and its header row + insert maxima + best scores for the all-reduce(MAX)
+static int shard_after_dp(miagpu_ctx* c, void** max_buf, int64_t* max_words) {
   cudaStream_t main = c->stream;
   const int64_t n = c->n;
-  c->sh_has_unique = has_unique;
-  if (!stats_done && !cut_launch_stats(c, 0, n, has_unique)) return 0;
-  MIAGPU_CUDA(cudaMemsetAsync(c->d_gaps.p, 0, (c->seq_len + 2) * sizeof(int32_t), main));
   int32_t* best = c->d_gaps.p + c->seq_len + 2;
   int32_t* hdr = best + MAX_READ + 1;
-  c->n_entries = 2 * n;
   if (c->fs_on) {
     // pointer state: this rank's slot count goes out with the header; the slots can only be numbered (and the entries take their
     // flags) once every rank's count is back -- miagpu_shard_fit.  The insert maxima need the entries' geometry only.
+    c->n_entries = 2 * n;
+    MIAGPU_CUDA(cudaMemsetAsync(c->d_gaps.p, 0, (c->seq_len + 2) * sizeof(int32_t), main));
     if (!fs_number(c)) return 0;
     if (n) {
       natural_entries_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_as_out.p, c->d_ae_out.p, c->d_nruns.p, c->d_runs.p,
@@ -2811,21 +2864,13 @@ static int shard_after_dp(miagpu_ctx* c, bool stats_done, bool has_unique, void*
       MIAGPU_CUDA(cudaGetLastError());
       c->launches++;
     }
-  } else {
-    MIAGPU_CUDA(cudaMemsetAsync(c->d_fs_cnt.p, 0, FS_CNT_WORDS * sizeof(int32_t), main));
+    if (!launch_gaps(c, main)) return 0;
+  } else if (!round_entries(c)) {
+    return 0;
   }
   shard_hdr2_kernel<<<1, 256, 0, main>>>(c->d_cstats.p, best, hdr, c->sh_world, c->sh_rank, (int)n, c->fs_on ? c->d_fs_cnt.p + FS_CNT_NSLOTS : nullptr);
   MIAGPU_CUDA(cudaGetLastError());
   c->launches++;
-  if (n && !c->fs_on) {
-    status_or_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_status.p, c->d_nruns.p, c->d_fs_cnt.p + FS_CNT_STATUS);
-    natural_entries_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_as_out.p, c->d_ae_out.p, c->d_nruns.p, c->d_runs.p,
-                                                                          c->d_status.p, c->seq_len, c->d_dropf.p, c->d_dropf.p, c->d_entries.p,
-                                                                          has_unique ? c->d_unique.p : nullptr);
-    MIAGPU_CUDA(cudaGetLastError());
-    c->launches += 2;
-  }
-  if (n && !launch_gaps(c)) return 0;
   if (max_buf) *max_buf = c->d_gaps.p;
   if (max_words) *max_words = c->seq_len + 2 + MAX_READ + 1 + (int64_t)c->sh_world * SHARD_HDR2;
   c->sh_phase = 1;
@@ -2854,20 +2899,10 @@ extern "C" int miagpu_shard_begin(miagpu_ctx* c, int world, int rank, int64_t n_
   if (c->fs_on && !c->h_unique.empty()) { set_error("miagpu_shard_begin: the pointer state in sharded rounds goes without the repeat filter"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   if (!shard_reserve_common(c, world, n_max)) return 0;
-  if (c->fs_on) {
-    if (!fs_reserve_round(c)) return 0;
-    c->fs_sharded = true;
-    fs_begin_round(c);
-  }
-  c->sh_world = world; c->sh_rank = rank; c->sh_nmax = n_max; c->sh_hard_cut = hard_cut; c->sh_cut_set = score_cut_set;
-  c->sh_slope = slope; c->sh_icpt = intercept; c->sh_fit = !score_cut_set && hard_cut <= 0; c->sh_host = false; c->sh_want_packed = false;
-  c->sh_phase = 0;
-  MIAGPU_CUDA(cudaEventRecord(c->ev[1], c->stream));
-  cut_init_kernel<<<1, 256, 0, c->stream>>>(c->d_cstats.p);
-  MIAGPU_CUDA(cudaGetLastError());
-  if (!realign_device(c, false)) return 0;
-  MIAGPU_CUDA(cudaEventRecord(c->ev[2], c->stream));
-  return shard_after_dp(c, false, !c->h_unique.empty(), max_buf, max_words);
+  c->sh_world = world; c->sh_rank = rank; c->sh_phase = 0;
+  c->round = RoundPolicy{hard_cut, score_cut_set, slope, intercept, !c->h_unique.empty()};
+  if (!round_start_resident(c, true) || !cut_launch_stats(c, 0, c->n, c->round.unique_best) || !shard_after_dp(c, max_buf, max_words)) return round_abort(c);
+  return 1;
 }
 
 extern "C" int miagpu_shard_begin_host(miagpu_ctx* c, int world, int rank, int64_t n_max, int64_t n, const uint8_t* bases,
@@ -2878,19 +2913,14 @@ extern "C" int miagpu_shard_begin_host(miagpu_ctx* c, int world, int rank, int64
   if (!shard_args(c, "miagpu_shard_begin_host", world, rank, n_max, n)) return 0;
   if (c->fs_on) { set_error("miagpu_shard_begin_host: the pointer state goes with resident reads (miagpu_shard_begin)"); return 0; }
   const Trace tr;
-  int C = 1;
   c->sh_phase = 0;
-  if (!host_round_front(c, "miagpu_shard_begin_host", n, bases, offsets, rc, as, ae, score, as_out, ae_out, abr, n_runs, status, seq_len,
-                        unique_best, true, dropped, tr, &C)) {
-    if (c->s_up) { cudaStreamSynchronize(c->s_down); cudaStreamSynchronize(c->s_up); }
-    return 0;
-  }
-  if (!shard_reserve_common(c, world, n_max)) return 0;
-  c->sh_world = world; c->sh_rank = rank; c->sh_nmax = n_max; c->sh_hard_cut = hard_cut; c->sh_cut_set = score_cut_set;
-  c->sh_slope = slope; c->sh_icpt = intercept; c->sh_fit = !score_cut_set && hard_cut <= 0; c->sh_host = true; c->sh_chunks = C;
-  // the flags of earlier rounds arrive on the upload stream: the entries (which take them) wait for them
-  MIAGPU_CUDA(cudaStreamWaitEvent(c->stream, c->xev[1], 0));
-  return shard_after_dp(c, true, unique_best != nullptr, max_buf, max_words);
+  const int C = host_round_front(c, "miagpu_shard_begin_host", n, bases, offsets, rc, as, ae, score, as_out, ae_out, abr, n_runs, status, seq_len,
+                                 unique_best, true, dropped, tr);
+  if (!C || !shard_reserve_common(c, world, n_max)) return round_abort(c);
+  c->sh_world = world; c->sh_rank = rank;
+  c->round = RoundPolicy{hard_cut, score_cut_set, slope, intercept, unique_best != nullptr, C};
+  if (!shard_after_dp(c, max_buf, max_words)) return round_abort(c);
+  return 1;
 }
 
 // After the all-reduce(MAX): this rank's part of the regression -- the sums of all ranks, the tables, the block records of the local
@@ -2901,7 +2931,6 @@ extern "C" int miagpu_shard_fit(miagpu_ctx* c, void** gather_send, void** gather
   MIAGPU_CUDA(cudaSetDevice(c->device));
   cudaStream_t main = c->stream, side = c->s_aux[2];
   const int64_t n = c->n, nb = c->sh_nb;
-  CutHost* H = c->h_cut;
   int32_t* best = c->d_gaps.p + c->seq_len + 2;
   int32_t* hdr = best + MAX_READ + 1;
   if (c->fs_on) {
@@ -2909,26 +2938,18 @@ extern "C" int miagpu_shard_fit(miagpu_ctx* c, void** gather_send, void** gather
     // slots, owners of the local slots (-1: another rank's), this round's pointers and the list of stale ones
     fs_base_kernel<<<1, 32, 0, main>>>(c->sh_world, c->sh_rank, hdr, SHARD_HDR2, c->d_fs_cnt.p);
     MIAGPU_CUDA(cudaMemsetAsync(c->d_slot_owner.p, 0xff, (size_t)c->fs_slot_cap * sizeof(int32_t), main));
-    if (!fs_entries(c, false)) return 0;
+    if (!fs_entries(c, false)) return round_abort(c);
     c->launches += 2;
   }
-  // insert-column layout from the reduced maxima
-  size_t tmp = 0;
-  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
-  if (!c->d_cub.reserve(tmp + 16)) return 0;
-  MIAGPU_CUDA(cub::DeviceScan::ExclusiveSum(c->d_cub.p, tmp, c->d_gaps.p, c->d_ins_off.p, c->seq_len + 1, main));
-  MIAGPU_CUDA(cudaMemcpyAsync(&H->total_ins, c->d_ins_off.p + c->seq_len, sizeof(int32_t), cudaMemcpyDeviceToHost, main));
-  MIAGPU_CUDA(cudaMemcpyAsync(H->fs_cnt, c->d_fs_cnt.p, sizeof(H->fs_cnt), cudaMemcpyDeviceToHost, main));
-  MIAGPU_CUDA(cudaEventRecord(c->aev[6], main));
-  c->launches += 2;
-  if (c->sh_fit) {
+  if (!round_layout(c)) return round_abort(c);          // from the reduced maxima
+  if (c->round.fit()) {
     uint32_t* send = c->d_sh_send.p;
     ShardBlockRec* recs = reinterpret_cast<ShardBlockRec*>(send);
     int32_t* pf_ids = reinterpret_cast<int32_t*>(send + (nb * sizeof(ShardBlockRec) + 3) / 4);
     uint32_t* pf_keys = reinterpret_cast<uint32_t*>(pf_ids + SHARD_PF_SLOTS + 8);
     shard_prep_kernel<<<1, 256, 0, main>>>(c->sh_world, c->sh_rank, hdr, best, c->d_cstats.p, c->d_ctab.p, c->d_sh_prep.p, pf_ids);
     CutSrc src{};
-    src.seq_len = c->d_seqlen.p; src.score = c->d_score.p; src.unique_best = c->sh_has_unique ? c->d_unique.p : nullptr;
+    src.seq_len = c->d_seqlen.p; src.score = c->d_score.p; src.unique_best = c->round.unique_best ? c->d_unique.p : nullptr;
     cut_approx_kernel<false><<<(unsigned)nb, CUT_THREADS, 0, main>>>(n, src, c->d_ctab.p, c->d_cblk.p);
     cut_prefix_kernel<<<1, CUT_PREFIX_THREADS, 0, main>>>(nb, c->d_cblk.p, c->d_sh_prep.p->start);
     cut_exact_kernel<false><<<(unsigned)nb, CUT_THREADS, 0, main>>>(n, src, c->d_ctab.p, c->d_cblk.p, pf_keys, pf_ids);
@@ -2936,29 +2957,14 @@ extern "C" int miagpu_shard_fit(miagpu_ctx* c, void** gather_send, void** gather
     MIAGPU_CUDA(cudaGetLastError());
     c->launches += 5;
   }
-  // the column planes: sized on the host from the layout (one short wait), accumulated beside the regression
-  MIAGPU_CUDA(cudaEventSynchronize(c->aev[6]));
-  if (H->fs_cnt[FS_CNT_STATUS]) {
-    cudaStreamSynchronize(main);
-    set_error("miagpu_shard_fit: local reads came back with status bits 0x%x (more than %d alignment runs, or a window no kernel takes)", H->fs_cnt[FS_CNT_STATUS], MAX_RUNS);
-    return 0;
-  }
-  // pointer state: stale pointers -> extra entries / patched smp parameters / frozen content, all of it local to this rank
-  if (c->fs_on && !fs_after_numbering(c, false, H->fs_cnt, &H->total_ins)) { cudaStreamSynchronize(main); return 0; }
-  c->n_cols = (int64_t)c->seq_len + H->total_ins;
-  // the planes are followed by nothing yet: the caller all-reduces exactly n_cols * NPLANE words
-  if (!c->d_acc.reserve(c->n_cols * NPLANE) || !c->d_called.reserve(c->n_cols + 16)) return 0;
-  MIAGPU_CUDA(cudaStreamWaitEvent(side, c->aev[6], 0));
-  MIAGPU_CUDA(cudaMemsetAsync(c->d_acc.p, 0, c->n_cols * NPLANE * sizeof(int32_t), side));
-  cudaStream_t keep = c->stream;
-  c->stream = side;                                    // launch_accumulate puts its kernels on c->stream
-  const int ok = launch_accumulate(c);
-  c->stream = keep;
-  if (!ok) return 0;
+  // the column planes (pointer state: stale pointers -> extra entries / patched smp parameters / frozen content, all of it local to
+  // this rank), accumulated on the side stream beside the regression.  The planes are followed by nothing yet: the caller
+  // all-reduces exactly n_cols * NPLANE words.
+  if (!round_planes(c, side) || !launch_accumulate(c, side)) return round_abort(c);
   MIAGPU_CUDA(cudaEventRecord(c->aev[7], side));
   if (gather_send) *gather_send = c->d_sh_send.p;
   if (gather_recv) *gather_recv = c->d_sh_recv.p;
-  if (gather_words) *gather_words = c->sh_fit ? c->sh_stride : 0;
+  if (gather_words) *gather_words = c->round.fit() ? c->sh_stride : 0;
   c->sh_phase = 2;
   return 1;
 }
@@ -2967,12 +2973,11 @@ extern "C" int miagpu_shard_cut(miagpu_ctx* c, double* slope_out, double* interc
   if (!c || c->sh_phase != 2) { set_error("miagpu_shard_cut: call miagpu_shard_fit first"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
   cudaStream_t main = c->stream;
-  const int64_t n = c->n, stride = c->sh_stride, nb = c->sh_nb;
+  const int64_t stride = c->sh_stride, nb = c->sh_nb;
   const int world = c->sh_world;
-  const bool fit = c->sh_fit;
   CutHost* H = c->h_cut;
-  double slope = c->sh_slope, intercept = c->sh_icpt;
-  if (fit) {
+  double slope = c->round.slope, intercept = c->round.intercept;
+  if (c->round.fit()) {
     // every rank's records, ids and the first SHARD_PF_FIRST key blocks in one strided copy; the other key blocks only if a rank used them
     const size_t pitch = (size_t)stride * sizeof(uint32_t);
     const size_t ids_at = ((size_t)nb * sizeof(ShardBlockRec) + 3) / 4 * 4;
@@ -2992,8 +2997,8 @@ extern "C" int miagpu_shard_cut(miagpu_ctx* c, double* slope_out, double* interc
     CutFit F;
     S.sx = H->prep.sx; S.sy = H->prep.sy; S.cnt = H->prep.cnt; S.bad = H->stats.bad == LLONG_MAX ? -1 : H->stats.bad;
     memcpy(S.best, H->stats.best, sizeof(S.best));
-    if (S.bad >= 0) { set_error("miagpu_shard_cut: seq_len of local read %lld out of range", (long long)S.bad); return 0; }
-    if (S.cnt <= 0) { set_error("miagpu_shard_cut: no read of any rank scores >= %d: nothing to fit", FIRST_ROUND_SCORE_CUTOFF); return 0; }
+    if (S.bad >= 0) { set_error("miagpu_shard_cut: seq_len of local read %lld out of range", (long long)S.bad); return round_abort(c); }
+    if (S.cnt <= 0) { set_error("miagpu_shard_cut: no read of any rank scores >= %d: nothing to fit", FIRST_ROUND_SCORE_CUTOFF); return round_abort(c); }
     cut_fit_tables(S, F);
     const int64_t nbt = (int64_t)world * nb;
     std::vector<ChainBlock> bxy(nbt), bxx(nbt);
@@ -3037,29 +3042,16 @@ extern "C" int miagpu_shard_cut(miagpu_ctx* c, double* slope_out, double* interc
     }, &ser1);
     if (missing) {
       set_error("miagpu_shard_cut: %d blocks of the regression's chains could not be proven and their keys did not travel (at most %d blocks per rank send keys; %s)", missing, SHARD_PF_SLOTS, first_missing);
-      return 0;
+      return round_abort(c);
     }
     c->cut_serial_blocks = ser0 + ser1;
-    c->sh_fetched = 0;
     cut_fit_slope(S, F, ssxy, ssxx, &slope, &intercept);
   }
   if (slope_out) *slope_out = slope;
   if (intercept_out) *intercept_out = intercept;
-  c->sh_slope = slope; c->sh_icpt = intercept;
-  // ---- flags of the local reads (cull_maln_from_fsdb, mia.c:452-470), sticky (H10); the reads this round drops leave the base columns
-  cut_thresholds(c->sh_hard_cut, slope, intercept, H->thr);
-  MIAGPU_CUDA(cudaMemcpyAsync(c->d_thr.p, H->thr, sizeof(H->thr), cudaMemcpyHostToDevice, main));
+  // flags of the local reads; with pointer state, every slot a local pointer reaches is local (miagpu_shard_fit)
   MIAGPU_CUDA(cudaStreamWaitEvent(main, c->aev[7], 0));                                // the accumulation of shard_fit
-  if (n && c->fs_on) {
-    if (!fs_flags_and_undo(c, false)) return 0;      // through the pointers; every slot a local pointer reaches is local (miagpu_shard_fit)
-  } else if (n) {
-    cut_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(n, c->d_seqlen.p, c->d_score.p, c->d_thr.p, c->d_dropf.p, nullptr, c->d_cstats.p,
-                                                                    c->sh_has_unique ? c->d_unique.p : nullptr, c->d_newly.p);
-    undo_kernel<<<(unsigned)((n + 255) / 256), 256, 0, main>>>(cons_params(c), n, c->d_newly.p, c->d_entries.p);
-    MIAGPU_CUDA(cudaGetLastError());
-    c->launches += 2;
-  }
-  MIAGPU_CUDA(cudaEventRecord(c->xev[2], main));
+  if (!round_flags(c, slope, intercept, false)) return round_abort(c);
   if (sum_buf) *sum_buf = c->d_acc.p;
   if (sum_words) *sum_words = c->n_cols * NPLANE;
   c->sh_phase = 3;
@@ -3070,38 +3062,17 @@ extern "C" int miagpu_shard_finish(miagpu_ctx* c, int cons_code, uint8_t* droppe
                                    int64_t* total_runs, int32_t* gaps_out, char* cons_out, int32_t* cons_len) {
   if (!c || c->sh_phase != 3) { set_error("miagpu_shard_finish: call miagpu_shard_cut first"); return 0; }
   MIAGPU_CUDA(cudaSetDevice(c->device));
-  cudaStream_t down = c->s_down;
-  const int64_t n = c->n;
   c->sh_phase = 0;
-  if (dropped && n) {
-    MIAGPU_CUDA(cudaStreamWaitEvent(down, c->xev[2], 0));
-    MIAGPU_CUDA(cudaMemcpyAsync(dropped, c->d_dropf.p, n, cudaMemcpyDeviceToHost, down));
-  }
-  c->cons_stage = 2;
-  const int launches = c->launches;
-  if (!miagpu_call(c, cons_code, gaps_out, nullptr, cons_out, cons_len)) { cudaStreamSynchronize(down); return 0; }
-  c->launches = launches + 1;
-  float ms_dp = 0;
-  if (!c->sh_host) MIAGPU_CUDA(cudaEventElapsedTime(&ms_dp, c->ev[1], c->ev[2]));
-  if (packed_runs || total_runs) {
+  if (!round_call(c, cons_code, dropped, gaps_out, cons_out, cons_len) || !round_end(c)) return round_abort(c);
+  if (packed_runs || total_runs) {                   // the round's launch count and times stand
+    const int launches = c->launches;
+    const float ms_kernels = c->ms_kernels, ms_d2h = c->ms_d2h;
     int64_t tot = 0;
-    const int l2 = c->launches;
-    if (!miagpu_get_runs_packed(c, nullptr, packed_runs, capacity, &tot)) { cudaStreamSynchronize(down); return 0; }
-    c->launches = l2 + 4;
+    if (!miagpu_get_runs_packed(c, nullptr, packed_runs, capacity, &tot)) return round_abort(c);
+    c->launches = launches + 4; c->ms_kernels = ms_kernels; c->ms_d2h = ms_d2h;
     if (total_runs) *total_runs = tot;
   }
-  MIAGPU_CUDA(cudaStreamSynchronize(down));
-  if (c->sh_host) {
-    MIAGPU_CUDA(cudaStreamSynchronize(c->s_up));
-    if (!host_round_stats(c, c->sh_chunks)) return 0;
-    c->misinc_stale = nullptr;
-    return 1;
-  }
-  c->ms_kernels = ms_dp;
-  c->ms_h2d = c->ms_d2h = 0;
-  MIAGPU_CUDA(cudaMemcpy(&c->n_fallback, c->d_meta.p + META_NFALL, 4, cudaMemcpyDeviceToHost));
-  if (c->fs_on) c->fs_prev_seq_len = c->seq_len;     // the geometry of this round's alignments, should the next round have to freeze one
-  c->misinc_stale = nullptr;
+  MIAGPU_CUDA(cudaStreamSynchronize(c->s_down));
   return 1;
 }
 
@@ -3119,7 +3090,7 @@ extern "C" int miagpu_shard_flags(miagpu_ctx* c, void** flag_buf, int64_t* bytes
 extern "C" int miagpu_last_cut_stats(miagpu_ctx* c, int64_t* serial_blocks, int64_t* fetched_blocks) {
   if (!c) { set_error("miagpu_last_cut_stats: no context"); return 0; }
   if (serial_blocks) *serial_blocks = c->cut_serial_blocks;
-  if (fetched_blocks) *fetched_blocks = c->sh_fetched;
+  if (fetched_blocks) *fetched_blocks = 0;
   return 1;
 }
 

@@ -29,13 +29,23 @@ def _separate(gpu, api, bases, off, rc, as_, ae, seq_len, sticky, unique_best=No
     return out, fit, drop, cons, gaps
 
 
-@pytest.mark.parametrize("n_reads,ref_len,seed", [(300, 1500, 3), (9000, 3000, 4), (120000, 6000, 5)])
-def test_iterate_resident_equals_separate_calls(gpu, n_reads, ref_len, seed):
+@pytest.mark.parametrize("n_reads,ref_len,seed,heavy", [(300, 1500, 3, 0.0), (9000, 3000, 4, 0.0), (120000, 6000, 5, 0.0), (20000, 3000, 6, 0.2)],
+                         ids=["300-1500-3", "9000-3000-4", "120000-6000-5", "20000-3000-6-heavy"])
+def test_iterate_resident_equals_separate_calls(gpu, n_reads, ref_len, seed, heavy):
     from mia_b200 import api
     ref, bases, off, rc, as_, ae = gpu_checks.make_case(n_reads, ref_len, seed=seed, divergence=0.02, indel_rate=0.004)
+    n = len(off) - 1
+    if heavy:
+        # a `heavy` share of the reads with a quarter of their bases substituted: low scores, no indels, few runs, no status bits.
+        # Round 1 then drops more than an eighth of the reads, so round 2 flags the entries before it accumulates the columns.
+        rng = np.random.default_rng(seed)
+        read_of = np.repeat(np.arange(n), np.diff(off))
+        sub = (rng.random(n) < heavy)[read_of] & (rng.random(len(bases)) < 0.25)
+        code = np.searchsorted(np.frombuffer(b"ACGT", np.uint8), bases[sub]) % 4
+        bases = bases.copy()
+        bases[sub] = np.frombuffer(b"ACGT", np.uint8)[(code + rng.integers(1, 4, len(code))) % 4]
     gpu.set_pssm(gpu_checks.load_pssm("onepass"))
     gpu.set_reference(ref, circular=1, with_rc=0)
-    n = len(off) - 1
     seq_len = np.diff(off).astype(np.int32)
     sticky = (np.arange(n) % 89 == 0).astype(np.uint8)
     out, fit, drop, cons, gaps = _separate(gpu, api, bases, off, rc, as_, ae, seq_len, sticky)
@@ -47,6 +57,8 @@ def test_iterate_resident_equals_separate_calls(gpu, n_reads, ref_len, seed):
     assert _bits(fit2[0]) == _bits(fit[0]) and _bits(fit2[1]) == _bits(fit[1]), (fit, fit2)
     assert (d2 == drop).all()
     assert cons2 == cons and (gaps2 == gaps).all()
+    if heavy:
+        assert int(((d2 == 1) & (sticky == 0)).sum()) * 8 > n
     # a second round on the same inputs: the flags are sticky on the device, nothing changes
     d3 = np.zeros(n, np.uint8)
     cons3, fit3, _ = gpu.iterate_resident(dropped=d3)
